@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- agent-steps/sec of the env-step + PPO-rollout hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -57,7 +57,14 @@ def parse_args():
     ap.add_argument('--epochs', type=int, default=4)
     ap.add_argument('--kernels-only', action='store_true', help='skip the PPO loop; report the per-kernel rooflines')
     ap.add_argument('--ref-horizon', type=int, default=8, help='bounded sample: env steps per reference-arm step')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed to DIR/<name>.npy (see dump_outputs)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.kernels_only):
+        ap.error('--dump-outputs needs the timed PPO steps of --impl b200')
+    return args
 
 
 def ppo_config(num_envs, horizon, device, seed=1, cuda_graph=True, minibatches=4, epochs=4, env='breakout'):
@@ -157,6 +164,46 @@ def timed_steps(data, cp, steps, world):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         dist.barrier()
     return float(ms.item())
+
+
+DUMP_ROWS = 1 << 16              # rollout rows sampled for the per-row arrays
+DUMP_OBS_BYTES = 32 << 20        # float32 bytes of sampled observation rows
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(data, out_dir):
+    """Write what the last PPO step handed its caller to out_dir/<name>.npy (float32, or float64 for statistics), so that
+    two builds run with the same arguments -- hence the same seeded inputs -- can be compared array by array:
+      param_<name>   the policy parameters after the update;
+      loss_<name>    the loss statistics of train(); stat_<name> the episode statistics of evaluate();
+      rows           the sampled rollout row positions (a fixed, seeded sample of DUMP_ROWS rows); <field> the rollout
+                     tensors of the Experience at those positions (actions, logprobs, rewards, dones, values,
+                     advantages, returns);
+      obs_rows, obs  an evenly spaced subset of `rows` and their observations (at most DUMP_OBS_BYTES)."""
+    exp = data.experience
+    out = {}
+    for name, p in data.policy.named_parameters():
+        out['param_' + name] = p.detach().float().cpu().numpy()
+    for k, v in data.losses.items():
+        out['loss_' + k] = np.float64(v)
+    for k, v in data.stats.items():
+        out['stat_' + k.replace('/', '_')] = np.float64(v)
+    b = exp.batch_size
+    rows = np.sort(np.random.default_rng(0).choice(b, min(b, DUMP_ROWS), replace=False))
+    idx = torch.as_tensor(rows, device=exp.obs.device)
+    out['rows'] = rows.astype(np.float64)
+    for k in ('actions', 'logprobs', 'rewards', 'dones', 'values', 'advantages', 'returns'):
+        out[k] = getattr(exp, k).index_select(0, idx).float().cpu().numpy()
+    k = min(len(rows), max(1, DUMP_OBS_BYTES // (4 * int(np.prod(exp.obs_shape)))))
+    sel = np.arange(k) * len(rows) // k
+    out['obs_rows'] = rows[sel].astype(np.float64)
+    out['obs'] = exp.obs.index_select(0, idx[torch.as_tensor(sel, device=idx.device)]).float().cpu().numpy()
+    total = sum(np.asarray(v).nbytes for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f'--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}')
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + '.npy'), np.asarray(v))
 
 
 def kernel_rooflines(data, args, peak_gbs, peak_src):
@@ -429,6 +476,8 @@ def run_b200(args):
     launches0, replays0, treplays0 = _native.lib().pb_launch_count(), data.graph_replays, data.train_graph_replays
     seg0 = getattr(data.train_segments, 'replayed_launches', 0)
     ms = timed_steps(data, cp, args.steps, world)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(data, args.dump_outputs)
     launches = ((_native.lib().pb_launch_count() - launches0) + (data.graph_replays - replays0) * data.graph_launches
                 + (data.train_graph_replays - treplays0) * data.train_graph_launches
                 + (getattr(data.train_segments, 'replayed_launches', 0) - seg0))
@@ -462,7 +511,7 @@ def run_b200(args):
             cp.evaluate(hdata); cp.train(hdata)
         hv = hdata.vecenv
         io0 = (hdata.io.h2d + hv.h2d_bytes, hdata.io.d2h + hv.d2h_bytes)
-        k_e2e = max(2, min(args.steps, 5))
+        k_e2e = args.steps
         ms_e = timed_steps(hdata, cp, k_e2e, world)
         io1 = (hdata.io.h2d + hv.h2d_bytes, hdata.io.d2h + hv.d2h_bytes)
         e2e = {'value': world * n * h * k_e2e / (ms_e * 1e-3), 'unit': UNIT, 'steps': k_e2e,

@@ -8,6 +8,8 @@ The reference cannot travel to the GPU box, so its outputs are committed here as
                     action tape (np.random.default_rng(0)); every recv() row (obs/reward/terminal/trunc/mask)
                     and every info dict.                        [vector.py:70-166, ocean.py:406-513]
   gae.npz           c_gae.compute_gae (the reference's Cython, built by pyximport) on seeded inputs.
+  c_gae_cases.npz   c_gae.compute_gae on the inputs of the tests that compare against it at larger sizes
+                    (``python tests/golden/generate.py c_gae_cases`` writes this file alone).
   experience_*.npz  clean_pufferl.Experience store -> sort_training_data -> compute_gae -> flatten_batch and
                     the per-minibatch advantage normalisation of clean_pufferl.train (torch CPU fp32).
 
@@ -84,10 +86,15 @@ def gae_inputs(n, seed, p_done=0.01):
     return dones, values, rewards
 
 
-def gen_gae():
+def load_c_gae():
     import pyximport
     pyximport.install(setup_args={'include_dirs': np.get_include()})
     from c_gae import compute_gae
+    return compute_gae
+
+
+def gen_gae():
+    compute_gae = load_c_gae()
     out = {}
     cases = [(1, 0, 0.01, 0.99, 0.95), (2, 1, 0.5, 0.99, 0.95), (7, 2, 0.3, 0.9, 0.8), (129, 3, 0.05, 0.99, 0.95),
              (8192, 0, 0.01, 0.99, 0.95), (8192, 4, 0.0, 1.0, 1.0), (4096, 5, 1.0, 0.99, 0.95),
@@ -101,6 +108,38 @@ def gen_gae():
     np.savez_compressed(os.path.join(HERE, 'gae.npz'), **out)
     print('gae cases', len(cases))
     return compute_gae
+
+
+# (n, p_done, gamma, lambda) of tests/test_oracle_golden.py::test_gae_oracle_vs_reference_compiled_c_gae
+C_GAE_CPU_CASES = [(2, 0.0, 0.99, 0.95), (1000, 0.02, 0.99, 0.95), (50000, 0.1, 0.9, 0.5), (4096, 1.0, 0.99, 0.95),
+                   (4096, 0.0, 1.0, 1.0)]
+# (h, n, p_done, gamma, lambda) of tests/test_gpu_gae.py::test_gae_vs_reference_compiled_c_gae
+C_GAE_GPU_CASES = [(128, 64, 0.02, 0.99, 0.95), (256, 1024, 0.01, 0.99, 0.95), (4096, 1, 0.05, 0.9, 0.8),
+                   (16, 333, 0.2, 1.0, 1.0), (128, 16384, 0.01, 0.99, 0.95)]
+C_GAE_SAMPLE = 16384
+
+
+def gen_c_gae_cases(compute_gae):
+    """c_gae.compute_gae on the inputs of the two reference-comparison tests above.  The CPU cases are stored whole (the
+    test is bit-exact); a GPU case longer than C_GAE_SAMPLE keeps a fixed, seeded sample of positions (gpu_*_idx)."""
+    out = {}
+    for n, p, gamma, lam in C_GAE_CPU_CASES:
+        d, v, r = gae_inputs(n, seed=n, p_done=p)
+        out[f'cpu_{n}_{p}_{gamma}_{lam}'] = np.asarray(compute_gae(d, v, r, gamma, lam))
+    for h, n, p, gamma, lam in C_GAE_GPU_CASES:
+        rng = np.random.default_rng(7 * h + n)                      # make_inputs of tests/test_gpu_gae.py
+        r = rng.standard_normal((h, n)).astype(np.float32)
+        v = rng.standard_normal((h, n)).astype(np.float32)
+        d = (rng.random((h, n)) < p).astype(np.float32)
+        r, v, d = (np.ascontiguousarray(x.T).reshape(-1) for x in (r, v, d))   # arrival [H, N] -> sorted e*H + t
+        adv = np.asarray(compute_gae(d, v, r, gamma, lam))
+        idx = np.arange(adv.size)
+        if adv.size > C_GAE_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(adv.size, C_GAE_SAMPLE, replace=False))
+        out[f'gpu_{h}x{n}_idx'] = idx.astype(np.int32)
+        out[f'gpu_{h}x{n}_adv'] = adv[idx]
+    np.savez_compressed(os.path.join(HERE, 'c_gae_cases.npz'), **out)
+    print('c_gae_cases', len(C_GAE_CPU_CASES), 'cpu +', len(C_GAE_GPU_CASES), 'gpu')
 
 
 def gen_experience(compute_gae):
@@ -234,8 +273,12 @@ def gen_lstm():
 
 
 if __name__ == '__main__':
+    if sys.argv[1:] == ['c_gae_cases']:       # only c_gae_cases.npz
+        gen_c_gae_cases(load_c_gae())
+        sys.exit()
     gen_squared()
     gen_squared_multiprocessing()
     cg = gen_gae()
     gen_experience(cg)
+    gen_c_gae_cases(cg)
     gen_lstm()

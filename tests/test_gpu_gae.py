@@ -111,21 +111,18 @@ def test_gae_argument_errors():
                                        _native.stream_ptr()))
 
 
-def test_gae_vs_reference_compiled_c_gae():
-    """pb_gae against the reference's OWN c_gae.pyx compiled here from /root/reference (oracle/_ref, built by
-    oracle/build_ref.py and shipped to the GPU box as a git-ignored artefact)."""
-    from oracle import build_ref
-    ref_mod = build_ref.load()
-    if ref_mod is None:
-        pytest.skip('oracle/_ref not built (no /root/reference at build time)')
+def test_gae_vs_reference_compiled_c_gae(golden):
+    """pb_gae against the reference's OWN c_gae.pyx: its outputs on these inputs are stored in c_gae_cases.npz by
+    generate.py, whole or, for the two larger cases, at a fixed sample of positions (idx)."""
+    g = golden('c_gae_cases')
     for h, n, p_done, gamma, lam in ((128, 64, 0.02, 0.99, 0.95), (256, 1024, 0.01, 0.99, 0.95), (4096, 1, 0.05, 0.9, 0.8),
                                      (16, 333, 0.2, 1.0, 1.0), (128, 16384, 0.01, 0.99, 0.95)):
         r, v, d = make_inputs(h, n, seed=7 * h + n, p_done=p_done)
         adv, ret = gae_device(r, v, d, gamma, lam)
         rs, vs, ds = (sorted_from_time_major(x) for x in (r, v, d))
-        ref = np.asarray(ref_mod.compute_gae(ds, vs, rs, gamma, lam))
+        idx, ref = g[f'gpu_{h}x{n}_idx'], g[f'gpu_{h}x{n}_adv']
         ref64 = ogae.compute_gae_f64(ds, vs, rs, gamma, lam)
-        gae_tolerance_check(adv, ref, ref64)
+        gae_tolerance_check(adv[idx], ref, ref64[idx])
 
 
 @pytest.mark.parametrize('h,n', [(128, 64), (128, 36), (256, 1024), (512, 40), (128, 16384)])

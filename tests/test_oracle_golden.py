@@ -124,15 +124,11 @@ def test_experience_validation_errors():
 
 @pytest.mark.parametrize('n,p_done,gamma,lam', [(2, 0.0, 0.99, 0.95), (1000, 0.02, 0.99, 0.95), (50000, 0.1, 0.9, 0.5),
                                                 (4096, 1.0, 0.99, 0.95), (4096, 0.0, 1.0, 1.0)])
-def test_gae_oracle_vs_reference_compiled_c_gae(n, p_done, gamma, lam):
-    """The oracle's C restatement against the reference's own c_gae.pyx compiled from /root/reference (oracle/_ref):
-    bit for bit, at sizes the golden file does not hold."""
-    from oracle import build_ref
-    ref_mod = build_ref.load()
-    if ref_mod is None:
-        pytest.skip('oracle/_ref not built (no /root/reference at build time)')
+def test_gae_oracle_vs_reference_compiled_c_gae(golden, n, p_done, gamma, lam):
+    """The oracle's C restatement against the reference's own c_gae.pyx (its outputs on these inputs are stored in
+    c_gae_cases.npz by generate.py): bit for bit, at sizes gae.npz does not hold."""
+    ref = golden('c_gae_cases')[f'cpu_{n}_{p_done}_{gamma}_{lam}']
     d, v, r = gae_inputs(n, seed=n, p_done=p_done)
-    ref = np.asarray(ref_mod.compute_gae(d, v, r, gamma, lam))
     got = ogae.compute_gae(d, v, r, gamma, lam)
     assert np.array_equal(ref.view(np.uint32), got.view(np.uint32))
 
