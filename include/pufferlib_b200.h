@@ -43,7 +43,7 @@ enum {
     PB_ERR_UNSUPPORTED = -4
 };
 
-enum { PB_ENV_SQUARED = 0, PB_ENV_BREAKOUT = 1, PB_ENV_SNAKE = 2, PB_ENV_PONG = 3 };
+enum { PB_ENV_SQUARED = 0, PB_ENV_BREAKOUT = 1, PB_ENV_SNAKE = 2, PB_ENV_PONG = 3, PB_ENV_SPACES = 4 };
 enum { PB_DTYPE_F32 = 0, PB_DTYPE_U8 = 1 };
 
 typedef struct pb_env pb_env; /* opaque: N env instances resident on one GPU */
@@ -58,7 +58,8 @@ typedef struct {
                                  SQUARED : [0]=distance_to_target (default 3; ocean/environment.py:28)
                                  BREAKOUT: [0]=max_ticks (default 4096)
                                  SNAKE   : [0]=max_ticks (default 1024)
-                                 PONG    : [0]=max_score (default 5) [1]=max_ticks (default 4096) */
+                                 PONG    : [0]=max_score (default 5) [1]=max_ticks (default 4096)
+                                 SPACES  : none */
 } pb_env_config;
 
 typedef struct {
@@ -66,7 +67,7 @@ typedef struct {
     int32_t obs_ndim;
     int32_t obs_shape[4];
     int64_t obs_bytes;    /* bytes of one agent's observation (O) */
-    int32_t num_actions;  /* Discrete(n) */
+    int32_t num_actions;  /* Discrete(n); 0 for MultiDiscrete kinds (pb_env_action_nvec) */
     int32_t num_envs;
     float obs_low, obs_high; /* Box bounds */
 } pb_env_info;
@@ -99,15 +100,19 @@ uint64_t pb_launch_count(void);
 int pb_env_create(const pb_env_config* cfg, pb_env** out);
 int pb_env_destroy(pb_env* env);
 int pb_env_get_info(const pb_env* env, pb_env_info* out);
+/* MultiDiscrete action space of the kind (emulation.py:115-120 turns a Dict / Tuple of Discrete into MultiDiscrete):
+ * nvec_out[0..n_heads) = head sizes, the rest of the 8 entries 0.  Discrete kinds report n_heads = 0. */
+int pb_env_action_nvec(const pb_env* env, int32_t* nvec_out /*[8]*/, int32_t* n_heads_out);
 
 /* vector.py:112-135: (re)seed env i with seed + env_index_offset + i (make_seeds, vector.py:639-641), reset it and
  * write the reset rows (r=0, terminal=False, truncation=False, mask=True; emulation.py:187-192). */
 int pb_env_reset(pb_env* env, uint64_t seed, const pb_env_out* out, void* stream);
 
 /* vector.py:137-156: envs whose previous row was terminal reset (action ignored, reset row written), all others
- * step with actions[e] (int64, Discrete).  PB_ERR_STATE before the first reset.  `actions` is validated on the
- * device only by clamping into [0, num_actions) -- the host layer does the reference's first-send
- * action_space.contains check (vector.py:36-39). */
+ * step with actions[e] (int64, Discrete) or actions[e][0..n_heads) (int64 [N][n_heads], MultiDiscrete kinds).
+ * PB_ERR_STATE before the first reset.  `actions` is validated on the device only by clamping (each column) into
+ * [0, num_actions) / [0, nvec[h]) -- the host layer does the reference's first-send action_space.contains check
+ * (vector.py:36-39). */
 int pb_env_step(pb_env* env, const int64_t* actions, const pb_env_out* out, void* stream);
 
 /* Snake step kernel variant for A/B measurements: lanes per env, 4 (default) or 16 (round 1); bit-identical results. */
@@ -218,6 +223,30 @@ int pb_ppo_loss(const float* logits, int64_t logits_stride, const float* value, 
                 const float* old_values, int64_t m, int32_t n_act, float clip_coef, int32_t clip_vloss,
                 float vf_clip_coef, float vf_coef, float ent_coef, float* grad_logits, int64_t grad_logits_stride,
                 float* grad_value, int64_t grad_value_stride, double* stats8, void* stream);
+
+/* -- MultiDiscrete heads (sampling + PPO loss) ----------------------------------------------------------------------
+ * pb_sample_logits_multi replaces sample_logits (pufferlib/frameworks/cleanrl.py:25-47) for a LIST of logits, one per
+ * head of a MultiDiscrete space (models.Default's decoder ModuleList, pufferlib/models.py:29-38, 57-59), when sampling:
+ * per head logsumexp and an inverse-CDF draw on the counter-based uniform of (seed, offset + *offset_dev, row, head);
+ * actions [n][n_heads] int64, logprob = sum over heads, entropy = sum over heads; the optional row stores are those of
+ * pb_sample_logits (actions_row is [n][n_heads]).  The head term of the RNG key vanishes for head 0, so nvec = {k}
+ * reproduces pb_sample_logits bit for bit.  The logits of one row are the heads' columns one after another, logits_stride
+ * floats apart (the packed [M, 8] head output: all heads | value | zero padding).  nvec_host: HOST array of n_heads
+ * (<= 16) sizes with sum <= 64.
+ * pb_ppo_loss_multi is pb_ppo_loss (the loss block of clean_pufferl.py:202-238) with newlogprob = sum_h normalized_h[a_h]
+ * and entropy = sum_h H_h: same six fp64 statistics, ATen tie rules and gradient layout (gradient columns follow the
+ * logit columns; a packed [m][8] gradient row -- grad_value == grad_logits + sum(nvec), both strides 8 -- is written
+ * whole, zero padding included).  actions: [m][n_heads] int64, clamped per head into [0, nvec[h]). */
+int pb_sample_logits_multi(const float* logits, int64_t logits_stride, int64_t n, const int32_t* nvec_host, int32_t n_heads,
+                           uint64_t seed, uint64_t offset, const uint64_t* offset_dev, int64_t* actions, float* logprobs,
+                           float* entropies, const float* value, int64_t value_stride, float* values_row,
+                           float* logprobs_row, int64_t* actions_row, void* stream);
+int pb_ppo_loss_multi(const float* logits, int64_t logits_stride, const float* value, int64_t value_stride,
+                      const int64_t* actions, const float* old_logprobs, const float* advantages, const float* returns,
+                      const float* old_values, int64_t m, const int32_t* nvec_host, int32_t n_heads, float clip_coef,
+                      int32_t clip_vloss, float vf_clip_coef, float vf_coef, float ent_coef, float* grad_logits,
+                      int64_t grad_logits_stride, float* grad_value, int64_t grad_value_stride, double* stats8,
+                      void* stream);
 
 /* -- fused rollout-time policy step --------------------------------------------------------------------------------
  * For models.Default with 128 input features and 128 hidden units (pufferlib/models.py:12-62): encoder Linear + ReLU,

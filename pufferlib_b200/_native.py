@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.environ.get('PUFFERLIB_B200_SO', os.path.join(HERE, 'libpuffer_b200.so'))   # override: debug builds
 
 PB_OK, PB_ERR_INVALID, PB_ERR_CUDA, PB_ERR_STATE, PB_ERR_UNSUPPORTED = 0, -1, -2, -3, -4
-ENV_KINDS = {'squared': 0, 'breakout': 1, 'snake': 2, 'pong': 3}
+ENV_KINDS = {'squared': 0, 'breakout': 1, 'snake': 2, 'pong': 3, 'spaces': 4}
 DTYPE_F32, DTYPE_U8 = 0, 1
 
 
@@ -56,6 +56,7 @@ SIGNATURES = {
     'pb_env_create': (C.c_int, [C.POINTER(EnvConfig), C.POINTER(C.c_void_p)]),
     'pb_env_destroy': (C.c_int, [C.c_void_p]),
     'pb_env_get_info': (C.c_int, [C.c_void_p, C.POINTER(EnvInfo)]),
+    'pb_env_action_nvec': (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     'pb_env_reset': (C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(EnvOut), C.c_void_p]),
     'pb_env_step': (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(EnvOut), C.c_void_p]),
     'pb_env_episode_rows': (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
@@ -77,6 +78,11 @@ SIGNATURES = {
     'pb_ppo_loss': (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 5 + [C.c_int64, C.c_int32,
                     C.c_float, C.c_int32, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_int64, C.c_void_p,
                     C.c_int64, C.c_void_p, C.c_void_p]),
+    'pb_sample_logits_multi': (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(C.c_int32), C.c_int32, C.c_uint64,
+                                         C.c_uint64] + [C.c_void_p] * 5 + [C.c_int64] + [C.c_void_p] * 3 + [C.c_void_p]),
+    'pb_ppo_loss_multi': (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64] + [C.c_void_p] * 5 +
+                          [C.c_int64, C.POINTER(C.c_int32), C.c_int32, C.c_float, C.c_int32, C.c_float, C.c_float, C.c_float,
+                           C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     'pb_policy_mlp_sample': (C.c_int, [C.c_void_p, C.c_int64] + [C.c_void_p] * 4 + [C.c_int64, C.c_int32, C.c_int32,
                              C.c_int32, C.c_uint64] + [C.c_void_p] * 6 + [C.c_void_p]),
     'pb_mlp_tail_workspace_bytes': (C.c_size_t, [C.c_int64, C.c_int32]),

@@ -150,6 +150,75 @@ class _FusedPPOLoss(torch.autograd.Function):
                 None)
 
 
+class _FusedPPOLossMulti(torch.autograd.Function):
+    """_FusedPPOLoss for a MultiDiscrete space (pb_ppo_loss_multi): `logits` holds every head's columns, head after head
+    ([M, sum(nvec)], or the packed [M, 8] head output with the value in column sum(nvec) when packed).  The gradient
+    comes back in the same layout, so the packed form hands ONE [M, 8] gradient to pb_mlp_tail_backward."""
+
+    @staticmethod
+    def forward(ctx, logits, value, actions, old_logprobs, adv, returns, old_values, cfg, nvec, packed):
+        clip_coef, clip_vloss, vf_clip_coef, vf_coef, ent_coef = cfg
+        total, m = sum(nvec), logits.shape[0]
+        if logits.stride(1) != 1 or logits.dtype != torch.float32:
+            logits = logits.float().contiguous()
+        grad = torch.empty_like(logits)
+        if packed:
+            l_ptr, v_ptr, v_stride = logits.data_ptr(), logits.data_ptr() + 4 * total, logits.stride(0)
+            grad_value = None
+            gv_ptr, gv_stride = grad.data_ptr() + 4 * total, grad.stride(0)
+            if grad.shape[1] != 8:          # the kernel writes whole rows only for [M, 8]
+                grad.zero_()
+        else:
+            v2 = value.reshape(m, -1)
+            l_ptr, v_ptr, v_stride = logits.data_ptr(), v2.data_ptr(), v2.stride(0)
+            grad_value = torch.empty(m, dtype=torch.float32, device=logits.device)
+            gv_ptr, gv_stride = grad_value.data_ptr(), 1
+            ctx.value_shape = value.shape
+        stats = torch.empty(8, dtype=torch.float64, device=logits.device)
+        cp = C.c_void_p
+        nv = (C.c_int32 * len(nvec))(*nvec)
+        _native.check(_native.lib().pb_ppo_loss_multi(
+            cp(l_ptr), logits.stride(0), cp(v_ptr), v_stride,
+            _native.ptr(actions.reshape(m, len(nvec)).contiguous()), _native.ptr(old_logprobs.reshape(-1).contiguous()),
+            _native.ptr(adv.reshape(-1).contiguous()), _native.ptr(returns.reshape(-1).contiguous()),
+            _native.ptr(old_values.reshape(-1).contiguous()), m, nv, len(nvec), C.c_float(clip_coef),
+            int(bool(clip_vloss)), C.c_float(vf_clip_coef), C.c_float(vf_coef), C.c_float(ent_coef), cp(grad.data_ptr()),
+            grad.stride(0), cp(gv_ptr), gv_stride, _native.ptr(stats), _native.stream_ptr()))
+        ctx.packed = packed
+        ctx.save_for_backward(grad, *(() if grad_value is None else (grad_value,)))
+        means = stats[:6] / m
+        means[1] *= 0.5
+        loss = (means[0] - ent_coef * means[2] + vf_coef * means[1]).float()
+        return loss, means.float()
+
+    @staticmethod
+    def backward(ctx, g_loss, g_stats):
+        none = (None,) * 8
+        if ctx.packed:
+            (grad,) = ctx.saved_tensors
+            return (g_loss * grad, None) + none
+        grad, grad_value = ctx.saved_tensors
+        return (g_loss * grad, (g_loss * grad_value).view(ctx.value_shape)) + none
+
+
+def _loss_cfg(config):
+    return (float(config.clip_coef), bool(config.clip_vloss), float(config.vf_clip_coef), float(config.vf_coef),
+            float(config.ent_coef))
+
+
+def fused_ppo_loss_multi(logits, value, actions, old_logprobs, adv, returns, old_values, config):
+    """fused_ppo_loss for a list of head logits (MultiDiscrete); actions [M, k]."""
+    nvec = [lg.shape[1] for lg in logits]
+    return _FusedPPOLossMulti.apply(torch.cat(logits, dim=1), value, actions, old_logprobs, adv, returns, old_values,
+                                    _loss_cfg(config), nvec, False)
+
+
+def fused_ppo_loss_packed_multi(out, nvec, actions, old_logprobs, adv, returns, old_values, config):
+    """fused_ppo_loss_packed for a MultiDiscrete models.Default: out = [M, 8] (all heads | value | zero padding)."""
+    return _FusedPPOLossMulti.apply(out, None, actions, old_logprobs, adv, returns, old_values, _loss_cfg(config),
+                                    list(nvec), True)
+
+
 def fused_ppo_loss(logits, value, actions, old_logprobs, adv, returns, old_values, config):
     """-> (loss, stats) with stats = [pg_loss, v_loss, entropy, old_approx_kl, approx_kl, clipfrac] (detached)."""
     cfg = (float(config.clip_coef), bool(config.clip_vloss), float(config.vf_clip_coef), float(config.vf_coef),
@@ -220,6 +289,8 @@ class _DefaultMLPUpdate:
                                                             torch.distributed.is_initialized()) else 1
             if world > 1:
                 return False      # opt-out: ranks > 1 on the autograd + GradBucket (NCCL) path
+        if not isinstance(model.decoder, torch.nn.Linear):
+            return False          # MultiDiscrete heads: the fused update kernel and this chain handle one Discrete head
         n_act, hid = model.decoder.weight.shape
         if hid != 128 or n_act > 7 or model.encoder.weight.dtype != torch.float32 or not model.encoder.weight.is_cuda:
             return False
@@ -459,8 +530,9 @@ class Experience:
             minibatch_size = batch_size
         if cpu_offload:
             raise NotImplementedError('cpu_offload: the B200 rollout is device-resident by design')
-        if len(tuple(atn_shape)) != 0:
-            raise NotImplementedError('only Discrete action spaces are on the device path')
+        atn_shape = tuple(atn_shape)
+        if len(atn_shape) > 1:
+            raise NotImplementedError('only Discrete and MultiDiscrete action spaces are on the device path')
         obs_dtype = numpy_to_torch_dtype_dict[np.dtype(obs_dtype)]
         dev = torch.device(device)
         if dev.type != 'cuda':
@@ -468,7 +540,9 @@ class Experience:
         self.device = dev
         z = dict(device=dev)
         self.obs = torch.zeros(batch_size, *obs_shape, dtype=obs_dtype, **z)
-        self.actions = torch.zeros(batch_size, dtype=torch.int64, **z)
+        self.actions = torch.zeros(batch_size, *atn_shape, dtype=torch.int64, **z)     # clean_pufferl.py:392
+        self.atn_shape = atn_shape
+        self.atn_row_bytes = 8 * int(np.prod(atn_shape, dtype=np.int64))
         self.logprobs = torch.zeros(batch_size, **z)
         self.rewards = torch.zeros(batch_size, **z)
         self.dones = torch.zeros(batch_size, **z)
@@ -506,7 +580,7 @@ class Experience:
         shape3 = (nm, self.minibatch_rows, bptt_horizon)
         self._b_obs = None        # [nm, minibatch_rows, bptt, *obs]: allocated by the first flatten_batch() that gathers
         self._slabs = None        # zero-copy minibatch form (flatten_batch_slabs)
-        self.b_actions = torch.zeros(shape3, dtype=torch.int64, **z)
+        self.b_actions = torch.zeros(*shape3, *atn_shape, dtype=torch.int64, **z)
         self.b_logprobs = torch.zeros(shape3, **z)
         self.b_dones = torch.zeros(shape3, **z)
         self.b_values = torch.zeros(nm, mb, **z)
@@ -583,18 +657,23 @@ class Experience:
             self.rewards[ptr:end] = torch.as_tensor(reward).to(self.device, torch.float32)
             self.dones[ptr:end] = torch.as_tensor(done).to(self.device, torch.float32)
         if isinstance(value, torch.Tensor) and value.data_ptr() == self.values.data_ptr() + ptr * 4 and \
-                isinstance(action, torch.Tensor) and action.data_ptr() == self.actions.data_ptr() + ptr * 8 and \
+                isinstance(action, torch.Tensor) and action.data_ptr() == self.actions.data_ptr() + ptr * self.atn_row_bytes and \
                 logprob.data_ptr() == self.logprobs.data_ptr() + ptr * 4:
             self.ptr = end          # the fused sampling epilogue already wrote value / logprob / action in place
             self.step += 1
             return
         value = value.reshape(-1).to(self.device, torch.float32).contiguous()
         logprob = logprob.reshape(-1).to(self.device, torch.float32).contiguous()
-        action = torch.as_tensor(action).reshape(-1).to(self.device, torch.int64).contiguous()
+        action = torch.as_tensor(action).reshape(n, *self.atn_shape).to(self.device, torch.int64).contiguous()
+        multi = len(self.atn_shape) > 0
         _native.check(lib.pb_rollout_store(
-            _native.ptr(value), _native.ptr(logprob), _native.ptr(action),
+            _native.ptr(value), _native.ptr(logprob), None if multi else _native.ptr(action),
             C.c_void_p(self.values.data_ptr() + ptr * 4), C.c_void_p(self.logprobs.data_ptr() + ptr * 4),
-            C.c_void_p(self.actions.data_ptr() + ptr * 8), n, s))
+            None if multi else C.c_void_p(self.actions.data_ptr() + ptr * 8), n, s))
+        if multi:               # [n, k] action rows: one row copy of 8k bytes each
+            _native.check(lib.pb_copy_rows(_native.ptr(action), self.atn_row_bytes,
+                                           C.c_void_p(self.actions.data_ptr() + ptr * self.atn_row_bytes),
+                                           self.atn_row_bytes, self.atn_row_bytes, n, s))
         self.ptr = end
         self.step += 1
 
@@ -677,11 +756,17 @@ class Experience:
         adv = self.advantages if advantages is None else advantages
         n, h = self.num_envs, self.horizon
         lib, s = _native.lib(), _native.stream_ptr()
+        multi = len(self.atn_shape) > 0
         _native.check(lib.pb_flatten_batch(
-            _native.ptr(self.actions), _native.ptr(self.logprobs), _native.ptr(self.dones), _native.ptr(self.values),
-            _native.ptr(adv), _native.ptr(self.b_actions), _native.ptr(self.b_logprobs), _native.ptr(self.b_dones),
+            None if multi else _native.ptr(self.actions), _native.ptr(self.logprobs), _native.ptr(self.dones),
+            _native.ptr(self.values), _native.ptr(adv), None if multi else _native.ptr(self.b_actions),
+            _native.ptr(self.b_logprobs), _native.ptr(self.b_dones),
             _native.ptr(self.b_values), _native.ptr(self.b_advantages), _native.ptr(self.b_returns),
             _native.ptr(self.returns), n, h, self.num_minibatches, self.minibatch_rows, self.bptt_horizon, s))
+        if multi:               # b_actions [nm, rows, bptt, k] = actions[b_idxs]: the observation gather on 8k-byte rows
+            _native.check(lib.pb_minibatch_gather(
+                _native.ptr(self.actions), _native.ptr(self.b_actions), self.atn_row_bytes, n, h, self.num_minibatches,
+                self.minibatch_rows, self.bptt_horizon, 0, self.num_minibatches, s))
         _native.check(lib.pb_minibatch_gather(
             _native.ptr(self.obs), _native.ptr(self.b_obs), self.obs_row_bytes, n, h, self.num_minibatches,
             self.minibatch_rows, self.bptt_horizon, 0, self.num_minibatches, s))
@@ -705,12 +790,13 @@ class Experience:
             z = dict(device=self.device)
             mb = self.minibatch_size
             self._slabs = pufferlib_b200.namespace(
-                actions=torch.zeros(nm, mb, dtype=torch.int64, **z), logprobs=torch.zeros(nm, mb, **z),
+                actions=torch.zeros(nm, mb, *self.atn_shape, dtype=torch.int64, **z), logprobs=torch.zeros(nm, mb, **z),
                 values=torch.zeros(nm, mb, **z), advantages=torch.zeros(nm, mb, **z), returns=torch.zeros(nm, mb, **z),
                 advantages_normalized=torch.zeros(nm, mb, **z))
         sl = self._slabs
         for dst, src in ((sl.actions, self.actions), (sl.logprobs, self.logprobs), (sl.values, self.values)):
-            dst.view(nm, g_, r_).copy_(src.view(g_, nm, r_).transpose(0, 1))
+            tail = tuple(src.shape[1:])          # (k,) for MultiDiscrete actions
+            dst.view(nm, g_, r_, *tail).copy_(src.view(g_, nm, r_, *tail).transpose(0, 1))
         sl.advantages.view(nm, g_, bptt, n).copy_(adv.view(n, g_, nm, bptt).permute(2, 1, 3, 0))   # sorted -> slab-major
         torch.add(sl.advantages, sl.values, out=sl.returns)
         torch.add(adv, self.values, out=self.returns)            # returns_np of clean_pufferl.py:476 (sorted + arrival)
@@ -805,9 +891,12 @@ def create(config, vecenv, policy, optimizer=None, wandb=None):
         io=pufferlib_b200.namespace(h2d=0, d2h=0), graph_state=0, rollout_graph=None, graph_steps=0,
         graph_launches=0, graph_replays=0, train_graph_state=0, train_graph=None, train_result=None, train_graph_launches=0, train_graph_replays=0, train_segments=None, train_acc=None, own_optimizer=own_optimizer, manual_update=None,
         fused_rows=bool(getattr(policy, 'fused_sample', False)) and hasattr(vecenv, 'bind_rollout'),
-        # one-kernel PPO loss (pb_ppo_loss): needs a wrapper exposing .policy(obs) -> (logits, value), one Discrete head
+        # one-kernel PPO loss (pb_ppo_loss, or pb_ppo_loss_multi for MultiDiscrete heads): needs a wrapper exposing
+        # .policy(obs) -> (logits, value)
         fused_loss=bool(getattr(config, 'fused_loss', True)) and hasattr(policy, 'policy')
-        and not hasattr(policy, 'lstm') and len(tuple(vecenv.single_action_space.shape)) == 0,
+        and not hasattr(policy, 'lstm') and len(tuple(vecenv.single_action_space.shape)) <= 1,
+        action_nvec=([int(x) for x in vecenv.single_action_space.nvec]
+                     if len(tuple(vecenv.single_action_space.shape)) == 1 else None),
     )
 
 
@@ -1096,7 +1185,14 @@ def _train_device_part(data, seg=None):
                 _, newlogprob, entropy, newvalue = data.policy(obs.reshape(-1, *obs_shape), action=atn)
 
         with profile.train_misc:
-            if fused:
+            if fused and data.action_nvec is not None:
+                if packed is not None:
+                    loss, st = fused_ppo_loss_packed_multi(packed[0], data.action_nvec, atn, log_probs, adv, ret, val,
+                                                           config)
+                else:
+                    loss, st = fused_ppo_loss_multi(logits, newvalue, atn, log_probs, adv, ret, val, config)
+                pg_loss, v_loss, entropy_loss, old_approx_kl, approx_kl, clipfrac = st.unbind(0)
+            elif fused:
                 if packed is not None:
                     loss, st = fused_ppo_loss_packed(packed[0], packed[1], atn, log_probs, adv, ret, val, config)
                 else:

@@ -68,7 +68,7 @@ extern "C" int pb_env_create(const pb_env_config* cfg, pb_env** out) {
     PB_REQUIRE(cfg && out, PB_ERR_INVALID, "pb_env_create: null pointer");
     *out = nullptr;
     PB_REQUIRE(cfg->num_envs >= 1, PB_ERR_INVALID, "num_envs must be at least 1");  // vector.py:578-579
-    PB_REQUIRE(cfg->kind >= PB_ENV_SQUARED && cfg->kind <= PB_ENV_PONG, PB_ERR_INVALID, "unknown env kind %d",
+    PB_REQUIRE(cfg->kind >= PB_ENV_SQUARED && cfg->kind <= PB_ENV_SPACES, PB_ERR_INVALID, "unknown env kind %d",
                cfg->kind);
     int ndev = 0;
     PB_CUDA(cudaGetDeviceCount(&ndev));
@@ -85,6 +85,7 @@ extern "C" int pb_env_create(const pb_env_config* cfg, pb_env** out) {
             case PB_ENV_BREAKOUT: rc = pb_breakout_create(env); break;
             case PB_ENV_SNAKE: rc = pb_snake_create(env); break;
             case PB_ENV_PONG: rc = pb_pong_create(env); break;
+            case PB_ENV_SPACES: rc = pb_spaces_create(env); break;
         }
     }
     if (rc != PB_OK) {
@@ -110,6 +111,13 @@ extern "C" int pb_env_destroy(pb_env* env) {
 extern "C" int pb_env_get_info(const pb_env* env, pb_env_info* out) {
     PB_REQUIRE(env && out, PB_ERR_INVALID, "pb_env_get_info: null pointer");
     *out = env->info;
+    return PB_OK;
+}
+
+extern "C" int pb_env_action_nvec(const pb_env* env, int32_t* nvec_out, int32_t* n_heads_out) {
+    PB_REQUIRE(env && nvec_out && n_heads_out, PB_ERR_INVALID, "pb_env_action_nvec: null pointer");
+    for (int h = 0; h < 8; ++h) nvec_out[h] = h < env->n_heads ? env->nvec[h] : 0;
+    *n_heads_out = env->n_heads;
     return PB_OK;
 }
 

@@ -37,6 +37,8 @@ struct pb_env {
     const void* const_trunc;
     const void* const_masks;
     bool write_const;
+    int32_t n_heads;         // MultiDiscrete kinds: action heads (0 = Discrete(info.num_actions)); actions are [N][n_heads]
+    int32_t nvec[8];
     void* kind;              // kind-specific state
 };
 
@@ -47,6 +49,7 @@ int pb_squared_create(pb_env* env);
 int pb_breakout_create(pb_env* env);
 int pb_snake_create(pb_env* env);
 int pb_pong_create(pb_env* env);
+int pb_spaces_create(pb_env* env);
 
 struct EpisodeAcc {
     double* ep_return;

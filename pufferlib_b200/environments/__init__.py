@@ -6,9 +6,18 @@ device-resident multi-env (the PufferEnv seam, pufferlib/environment.py:1-21).  
 ``b200_kind`` attribute (ours) or by name for the reference's own ``make_squared``
 (pufferlib/environments/ocean/environment.py:28-31), so the reference's creator can be passed unchanged.
 """
+import numpy as np
+
 from pufferlib_b200.exceptions import APIUsageError
 
-KNOWN_BY_NAME = {'make_squared': 'squared', 'make_breakout': 'breakout', 'make_snake': 'snake', 'make_pong': 'pong'}
+# kinds whose observation is a structured record: the np.dtype(align=True) of the native Dict space with gymnasium's
+# sorted keys (emulation.py:68-80), i.e. the `emulated_observation_dtype` of the reference's GymnasiumPufferEnv
+OBS_RECORD_DTYPE = {
+    'spaces': np.dtype([('flat', np.int8, (5,)), ('image', np.float32, (5, 5))], align=True),
+}
+
+KNOWN_BY_NAME = {'make_squared': 'squared', 'make_breakout': 'breakout', 'make_snake': 'snake', 'make_pong': 'pong',
+                 'make_spaces': 'spaces'}
 
 
 def resolve(creator, args, kwargs):
@@ -36,6 +45,8 @@ def resolve(creator, args, kwargs):
     elif kind == 'pong':
         iparam[0] = int(kwargs.pop('max_score', 0))
         iparam[1] = int(kwargs.pop('max_ticks', 0))
+    elif kind == 'spaces' and args:
+        raise APIUsageError('spaces: the env takes no arguments')
     if kwargs:
         raise APIUsageError(f'{kind}: unexpected env kwargs {sorted(kwargs)}')
     return kind, iparam

@@ -5,8 +5,10 @@ make_squared = _creator('squared')
 make_breakout = _creator('breakout')
 make_snake = _creator('snake')
 make_pong = _creator('pong')
+make_spaces = _creator('spaces')
 
-_CREATORS = {'squared': make_squared, 'breakout': make_breakout, 'snake': make_snake, 'pong': make_pong}
+_CREATORS = {'squared': make_squared, 'breakout': make_breakout, 'snake': make_snake, 'pong': make_pong,
+             'spaces': make_spaces}
 
 
 def env_creator(name='squared'):

@@ -26,13 +26,25 @@ def entropy(logits):
 
 
 def sample_logits(logits, action=None):
-    """Discrete head only (the configs of this path).  Returns (action, logprob, entropy)."""
-    normalized = logits - logits.logsumexp(dim=-1, keepdim=True)
+    """Returns (action, logprob, entropy).  `logits` is one tensor (Discrete) or a list with one tensor per head
+    (MultiDiscrete, the reference's semantics and shapes): action [N, k] (given actions are read as
+    action.view(N, -1).T), logprob and entropy summed over the heads."""
+    if isinstance(logits, torch.Tensor):
+        normalized = logits - logits.logsumexp(dim=-1, keepdim=True)
+        if action is None:
+            action = torch.multinomial(torch.softmax(normalized, dim=-1), 1).squeeze(-1)
+        else:
+            action = action.reshape(-1)
+        return action, log_prob(normalized, action), entropy(normalized)
+    normalized = [lg - lg.logsumexp(dim=-1, keepdim=True) for lg in logits]
     if action is None:
-        action = torch.multinomial(torch.softmax(normalized, dim=-1), 1).squeeze(-1)
+        action = torch.stack([torch.multinomial(torch.softmax(nl, dim=-1), 1).squeeze(-1) for nl in normalized])
     else:
-        action = action.reshape(-1)
-    return action, log_prob(normalized, action), entropy(normalized)
+        action = action.view(logits[0].shape[0], -1).T
+    assert len(normalized) == len(action)
+    logprob = torch.stack([log_prob(nl, a) for nl, a in zip(normalized, action)]).T.sum(1)
+    ent = torch.stack([entropy(nl) for nl in normalized]).T.sum(1)
+    return action.T, logprob, ent
 
 
 class Policy(torch.nn.Module):
@@ -59,6 +71,8 @@ class Policy(torch.nn.Module):
                 return fused
         logits, value = self.policy(x)
         if action is None and self.fused_sample and not torch.is_grad_enabled():
+            if not isinstance(logits, torch.Tensor):
+                return self._sample_fused_multi(logits, value, out)
             return self._sample_fused(logits, value, out)
         action, logprob, ent = sample_logits(logits, action)
         return action, logprob, ent, value
@@ -70,6 +84,8 @@ class Policy(torch.nn.Module):
         if not (hasattr(model, 'head_matrix') and getattr(model, 'fast_path', False) and x.is_cuda
                 and x.dtype == torch.float32):
             return None
+        if not isinstance(model.decoder, torch.nn.Linear):
+            return None           # the one-kernel policy step samples one Discrete head
         x2 = x.view(x.shape[0], -1)
         n_act, hid = model.decoder.weight.shape
         if x2.shape[1] != 128 or hid != 128 or n_act > 7 or x2.stride(1) != 1 or x2.stride(0) % 4 != 0:
@@ -116,6 +132,38 @@ class Policy(torch.nn.Module):
             _native.ptr(logits), logits.stride(0), n, a, C.c_uint64(self._seed), C.c_uint64(0),
             _native.ptr(self._counter), _native.ptr(actions), _native.ptr(logprob), _native.ptr(ent),
             _native.ptr(v2), v2.stride(0), rows[0], rows[1], rows[2], _native.stream_ptr()))
+        self._counter.add_(1)
+        return actions, logprob, ent, value_out
+
+    def _sample_fused_multi(self, logits, value, out=None):
+        """pb_sample_logits_multi on a list of head logits.  Heads that are consecutive column blocks of one row-major
+        tensor (models.Default's packed [M, 8] output) are read in place; otherwise they are concatenated once."""
+        n, dev = logits[0].shape[0], logits[0].device
+        nvec = [lg.shape[1] for lg in logits]
+        base, stride = logits[0], logits[0].stride(0)
+        in_place = base.dtype == torch.float32 and all(
+            lg.dtype == torch.float32 and lg.stride(1) == 1 and lg.stride(0) == stride
+            and lg.data_ptr() == base.data_ptr() + 4 * sum(nvec[:h]) for h, lg in enumerate(logits))
+        if not in_place:
+            base = torch.cat([lg.float() for lg in logits], dim=1).contiguous()
+            stride = base.stride(0)
+        if out is None:
+            actions = torch.empty(n, len(nvec), dtype=torch.int64, device=dev)
+            logprob = torch.empty(n, dtype=torch.float32, device=dev)
+            values_row = None
+            value_out = value
+        else:
+            value_out, logprob, actions = out
+            values_row = _native.ptr(value_out)
+        ent = torch.empty(n, dtype=torch.float32, device=dev)
+        if self._counter is None:
+            self._counter = torch.zeros(1, dtype=torch.int64, device=dev)
+        v2 = value.reshape(n, -1)
+        nv = (C.c_int32 * len(nvec))(*nvec)
+        _native.check(_native.lib().pb_sample_logits_multi(
+            _native.ptr(base), stride, n, nv, len(nvec), C.c_uint64(self._seed), C.c_uint64(0),
+            _native.ptr(self._counter), _native.ptr(actions), _native.ptr(logprob), _native.ptr(ent),
+            _native.ptr(v2), v2.stride(0), values_row, None, None, _native.stream_ptr()))
         self._counter.add_(1)
         return actions, logprob, ent, value_out
 

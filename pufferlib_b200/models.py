@@ -105,7 +105,14 @@ class Default(nn.Module):
     def __init__(self, env, hidden_size=128):
         super().__init__()
         self.encoder = nn.Linear(int(np.prod(env.single_observation_space.shape)), hidden_size)
-        self.decoder = layer_init(nn.Linear(hidden_size, env.single_action_space.n), std=0.01)
+        # MultiDiscrete: one decoder per head (models.py:29-38), state-dict keys decoder.0.weight, ...
+        nvec = getattr(env.single_action_space, 'nvec', None)
+        self.is_multidiscrete = nvec is not None
+        if self.is_multidiscrete:
+            self.nvec = [int(n) for n in nvec]
+            self.decoder = nn.ModuleList([layer_init(nn.Linear(hidden_size, n), std=0.01) for n in self.nvec])
+        else:
+            self.decoder = layer_init(nn.Linear(hidden_size, env.single_action_space.n), std=0.01)
         self.value_head = nn.Linear(hidden_size, 1)
         self.fast_path = True     # fused forward epilogues + pb_mlp_tail_backward (CUDA, hidden 128, <= 7 actions)
         self._head_cache = {}
@@ -115,19 +122,36 @@ class Default(nn.Module):
         train)."""
         self._head_cache.clear()
 
+    def decoder_params(self):
+        """(weight [n_logits, H], bias [n_logits]) of all action heads, head after head (a differentiable cat for a
+        MultiDiscrete decoder)."""
+        if self.is_multidiscrete:
+            return torch.cat([d.weight for d in self.decoder]), torch.cat([d.bias for d in self.decoder])
+        return self.decoder.weight, self.decoder.bias
+
+    @property
+    def n_logits(self):
+        return sum(self.nvec) if self.is_multidiscrete else self.decoder.out_features
+
+    def split_logits(self, logits):
+        """[M, n_logits] -> the reference's decode_actions output: one tensor, or a list of views per head."""
+        return list(logits.split(self.nvec, dim=1)) if self.is_multidiscrete else logits
+
     def head_matrix(self):
-        """(w_cat [8, H], b_cat [8]): n_act logit rows | value row | zero padding; cached under no_grad."""
+        """(w_cat [8, H], b_cat [8]): logit rows of every head | value row | zero padding; cached under no_grad."""
         cache = self._head_cache
-        key = (self.decoder.weight.data_ptr(), torch.cuda.is_current_stream_capturing())
+        w0 = self.decoder[0].weight if self.is_multidiscrete else self.decoder.weight
+        key = (w0.data_ptr(), torch.cuda.is_current_stream_capturing())
         if not torch.is_grad_enabled() and cache.get('key') == key:
             return cache['w'], cache['b']
-        n_act, hid = self.decoder.weight.shape
         with torch.no_grad():
-            w_cat = self.decoder.weight.new_zeros(8, hid)
-            w_cat[:n_act] = self.decoder.weight
+            w_dec, b_dec = self.decoder_params()
+            n_act, hid = w_dec.shape
+            w_cat = w_dec.new_zeros(8, hid)
+            w_cat[:n_act] = w_dec
             w_cat[n_act] = self.value_head.weight[0]
-            b_cat = self.decoder.weight.new_zeros(8)
-            b_cat[:n_act] = self.decoder.bias
+            b_cat = w_dec.new_zeros(8)
+            b_cat[:n_act] = b_dec
             b_cat[n_act] = self.value_head.bias[0]
         if not torch.is_grad_enabled():
             cache['key'], cache['w'], cache['b'] = key, w_cat, b_cat
@@ -148,19 +172,21 @@ class Default(nn.Module):
         return w
 
     def _fast_ok(self, x):
-        n_act, hid = self.decoder.weight.shape
-        return self.fast_path and x.is_cuda and hid == 128 and n_act + 1 <= 8 and not x.requires_grad
+        hid = self.encoder.out_features
+        return self.fast_path and x.is_cuda and hid == 128 and self.n_logits + 1 <= 8 and not x.requires_grad
 
     def forward_packed(self, observations):
-        """-> (out [M, 8], n_act) with logits = out[:, :n_act], value = out[:, n_act] (zero padding after), or None
-        when the fast path does not apply.  Lets the fused PPO loss hand back ONE [M, 8] gradient."""
+        """-> (out [M, 8], n_act) with logits = out[:, :n_act] (every head, head after head), value = out[:, n_act]
+        (zero padding after), or None when the fast path does not apply.  Lets the fused PPO loss hand back ONE [M, 8]
+        gradient."""
         x = observations.view(observations.shape[0], -1)
         if not self._fast_ok(x):
             return None
+        w_dec, b_dec = self.decoder_params()
         out = _DefaultMLPFunction.apply(x.float().contiguous(), self.encoder.weight, self.encoder.bias,
-                                        self.decoder.weight, self.decoder.bias, self.value_head.weight,
+                                        w_dec, b_dec, self.value_head.weight,
                                         self.value_head.bias, self._head_cache)
-        return out, self.decoder.weight.shape[0]
+        return out, self.n_logits
 
     def forward_packed_slabs(self, slabs):
         """forward_packed for a minibatch given as [G, R, features] row slabs (a strided view of the rollout
@@ -169,16 +195,17 @@ class Default(nn.Module):
             slabs = slabs.flatten(2)          # [G, R, *obs] -> [G, R, features] (a view: obs dims are contiguous)
         if slabs.dim() != 3 or not self._fast_ok(slabs) or slabs.stride(2) != 1 or slabs.stride(1) != slabs.shape[2]:
             return None
+        w_dec, b_dec = self.decoder_params()
         out = _DefaultMLPFunction.apply(slabs.float(), self.encoder.weight, self.encoder.bias,
-                                        self.decoder.weight, self.decoder.bias, self.value_head.weight,
+                                        w_dec, b_dec, self.value_head.weight,
                                         self.value_head.bias, self._head_cache)
-        return out, self.decoder.weight.shape[0]
+        return out, self.n_logits
 
     def forward(self, observations):
         packed = self.forward_packed(observations)
         if packed is not None:
             out, n_act = packed
-            return out[:, :n_act], out[:, n_act:n_act + 1]
+            return self.split_logits(out[:, :n_act]), out[:, n_act:n_act + 1]
         hidden, lookup = self.encode_observations(observations)
         return self.decode_actions(hidden, lookup)
 
@@ -190,12 +217,13 @@ class Default(nn.Module):
     def decode_actions(self, hidden, lookup, concat=True):
         # both heads out of ONE GEMM (same parameters, same math as two nn.Linear calls): the value head is a
         # 1-column GEMV that would otherwise re-read `hidden`
-        n_act = self.decoder.out_features
+        w_dec, b_dec = self.decoder_params()
+        n_act = w_dec.shape[0]
         pad = (-(n_act + 1)) % 8          # zero rows up to a multiple of 8 columns: keeps the aligned GEMM kernels
-        w = torch.cat([self.decoder.weight, self.value_head.weight, hidden.new_zeros(pad, hidden.shape[1])], dim=0)
-        b = torch.cat([self.decoder.bias, self.value_head.bias, hidden.new_zeros(pad)], dim=0)
+        w = torch.cat([w_dec, self.value_head.weight, hidden.new_zeros(pad, hidden.shape[1])], dim=0)
+        b = torch.cat([b_dec, self.value_head.bias, hidden.new_zeros(pad)], dim=0)
         out = torch.nn.functional.linear(hidden, w, b)
-        return out[:, :n_act], out[:, n_act:n_act + 1]
+        return self.split_logits(out[:, :n_act]), out[:, n_act:n_act + 1]
 
 
 class LSTMWrapper(nn.Module):

@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from pufferlib_b200 import _native, spaces
-from pufferlib_b200.environments import resolve
+from pufferlib_b200.environments import OBS_RECORD_DTYPE, resolve
 from pufferlib_b200.exceptions import APIUsageError
 from pufferlib_b200.namespace import Namespace, namespace
 
@@ -43,9 +43,14 @@ def send_precheck(vecenv, actions):
     if not vecenv.initialized:
         vecenv.initialized = True
         if isinstance(actions, torch.Tensor):
-            n = vecenv.single_action_space.n
-            ok = (actions.shape == (vecenv.num_agents,) and not actions.dtype.is_floating_point
-                  and bool(((actions >= 0) & (actions < n)).all()))
+            space = vecenv.single_action_space
+            if isinstance(space, spaces.MultiDiscrete):     # [N, k], column h in [0, nvec[h])
+                shape = (vecenv.num_agents, len(space))
+                bound = torch.as_tensor(space.nvec, device=actions.device)
+            else:
+                shape, bound = (vecenv.num_agents,), space.n
+            ok = (tuple(actions.shape) == shape and not actions.dtype.is_floating_point
+                  and bool(((actions >= 0) & (actions < bound)).all()))
         else:
             ok = vecenv.action_space.contains(np.asarray(actions))
         if not ok:
@@ -179,9 +184,16 @@ class B200:
         obs_shape = tuple(info.obs_shape[i] for i in range(info.obs_ndim))
         self.single_observation_space = spaces.Box(low=info.obs_low, high=info.obs_high, shape=obs_shape,
                                                    dtype=_NP_DTYPES[info.obs_dtype])
-        self.single_action_space = spaces.Discrete(info.num_actions)
+        nvec, heads = (C.c_int32 * 8)(), C.c_int32()
+        _native.check(lib.pb_env_action_nvec(self._handle, nvec, C.byref(heads)))
+        # MultiDiscrete kinds (emulation.py:115-120): actions are [N, k] int64 rows, column h in [0, nvec[h])
+        self.atn_heads = int(heads.value)
+        self.single_action_space = spaces.MultiDiscrete(list(nvec)[:self.atn_heads]) if self.atn_heads else \
+            spaces.Discrete(info.num_actions)
+        atn_shape = (num_envs, self.atn_heads) if self.atn_heads else (num_envs,)
+        self._atn_row_bytes = 8 * max(1, self.atn_heads)
         self.emulated = namespace(observation_dtype=self.single_observation_space.dtype,
-                                  emulated_observation_dtype=self.single_observation_space.dtype)
+                                  emulated_observation_dtype=OBS_RECORD_DTYPE.get(kind, self.single_observation_space.dtype))
         self.agents_per_batch = num_envs
         self.num_agents = num_envs
         self.action_space = joint_space(self.single_action_space, num_envs)
@@ -199,7 +211,7 @@ class B200:
                 masks=torch.ones(num_envs, dtype=torch.bool, device=self.device),
                 dones_f32=torch.zeros(num_envs, dtype=torch.float32, device=self.device),
             )
-            self._actions_dev = torch.zeros(num_envs, dtype=torch.int64, device=self.device)
+            self._actions_dev = torch.zeros(atn_shape, dtype=torch.int64, device=self.device)
         self.driver_env = _DriverEnv(self)
         # rollout binding (clean_pufferl.create): step outputs go straight into Experience rows
         self._rollout = None
@@ -212,7 +224,7 @@ class B200:
                 terminals=torch.zeros(num_envs, dtype=torch.bool).pin_memory(),
                 truncations=torch.zeros(num_envs, dtype=torch.bool).pin_memory(),
                 masks=torch.ones(num_envs, dtype=torch.bool).pin_memory(),
-                actions=torch.zeros(num_envs, dtype=torch.int64).pin_memory(),
+                actions=torch.zeros(atn_shape, dtype=torch.int64).pin_memory(),
             )
             self._host_np = namespace(**{k: v.numpy() for k, v in self._host.items()})
             with torch.cuda.device(self.device):
@@ -292,7 +304,7 @@ class B200:
                 row = self._cursor + 1
             for handle, lo, _ in self._shards:
                 out = self._env_out(row, lo)
-                _native.check(_native.lib().pb_env_step(handle, C.c_void_p(a.data_ptr() + 8 * lo), C.byref(out),
+                _native.check(_native.lib().pb_env_step(handle, C.c_void_p(a.data_ptr() + self._atn_row_bytes * lo), C.byref(out),
                                                         _native.stream_ptr()))
             if self._rollout is not None:
                 if row is None:
@@ -365,7 +377,7 @@ class B200:
                                                  _native.stream_ptr()))
         self._ev_act.record()
         self._act_pending = True
-        self.d2h_bytes += 8 * self.num_agents
+        self.d2h_bytes += self._atn_row_bytes * self.num_agents
         return self._host_np.actions
 
     def join_copies(self):
@@ -409,6 +421,8 @@ class B200:
         path, rollout bound to `experience` and standing at a rollout boundary, models.Default 128 -> 128 -> <= 4 actions
         behind a cleanrl.Policy with the fused sampler."""
         model = getattr(policy, 'policy', None)
+        if not isinstance(self.single_action_space, spaces.Discrete):
+            return False          # the persistent kernel samples one Discrete head
         if not (self.kind == 'breakout' and not self.host_buffers and not self.exact_infos and len(self._shards) == 1
                 and self._rollout is experience and self._pending_own and self._cursor == 0 and self.flag == RECV
                 and self.num_agents % 128 == 0 and experience.ptr == 0 and experience.lstm_h is None):
