@@ -307,18 +307,15 @@ int pb_mlp_tail_backward(const float* dout, int64_t dout_stride, const float* w_
  *   returns      nullable: advantages (raw) + old_values is used (clean_pufferl.py:476-481)
  *   grad_flat    [128*128 + 8*128 + 128 + 8]: dW_enc | dW_heads | db_enc | db_heads  (what pb_clip_adam consumes)
  *   stats8       the six loss sums of pb_ppo_loss (zeroed here)
- *   dpre_out     null: dW_enc = dPre^T x is accumulated inside the kernel (MN-major UMMAs; x is loaded a second time in the
- *                SWIZZLE_128B_BASE32B layout the tensor core requires for transposed 32-bit operands).  Non-null: dPre
- *                [M][128] (slab-major rows) is written there instead and the dW_enc part of grad_flat is left to the caller
+ *   dpre_out     must be NULL (anything else returns PB_ERR_UNSUPPORTED): dW_enc = dPre^T x is always accumulated inside
+ *                the kernel, and dPre is never written to memory
  *   dbg_*        nullable dumps of relu(h) [M][128], dPre [M][128], dOut [M][8] for validation. */
 size_t pb_mlp_update_workspace_bytes(void);
-/* 1 = two x layouts per tile (K-major + MN-major TMA loads), 2 = one x layout, x^T formed on the tensor core */
-int pb_mlp_update_set_variant(int32_t variant);
-/* the reduce step of pb_mlp_update_fused also leaves the sum of squares of the gradient it wrote as pb_mlp_update_sumsq_parts()
- * doubles at byte pb_mlp_update_sumsq_offset() of the workspace (dW-in-kernel mode): input of pb_clip_adam_parts */
+/* the reduce step of pb_mlp_update_fused also leaves the sum of squares of the whole gradient it wrote as
+ * pb_mlp_update_sumsq_parts() doubles at byte pb_mlp_update_sumsq_offset() of the workspace: input of pb_clip_adam_parts */
 size_t pb_mlp_update_sumsq_offset(void);
 int32_t pb_mlp_update_sumsq_parts(void);
-/* profiling hook (variant 2): SM-clock stamps of tiles 8..11, [grid][18 warps][4][8] int64; NULL switches it off */
+/* profiling hook: SM-clock stamps of tiles 8..11, [grid][18 warps][4][8] int64; NULL switches it off */
 int pb_mlp_update_debug_clock(long long* buf);
 int pb_mlp_update_fused(const float* x, int64_t ldx, int64_t slab_rows, int64_t slab_stride_rows, int32_t n_slabs,
                         const float* w_enc, const float* b_enc, const float* w_heads, const float* b_heads,

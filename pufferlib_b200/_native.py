@@ -92,7 +92,6 @@ SIGNATURES = {
                                 [C.c_int32, C.c_uint64, C.c_void_p, C.c_void_p]),
     'pb_rollout_debug_buffers': (C.c_int, [C.c_void_p, C.c_void_p]),
     'pb_mlp_update_workspace_bytes': (C.c_size_t, []),
-    'pb_mlp_update_set_variant': (C.c_int, [C.c_int32]),
     'pb_mlp_update_debug_clock': (C.c_int, [C.c_void_p]),
     'pb_mlp_update_fused': (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32] + [C.c_void_p] * 10 +
                             [C.c_int64, C.c_int32, C.c_float, C.c_int32, C.c_float, C.c_float, C.c_float] + [C.c_void_p] * 3 +

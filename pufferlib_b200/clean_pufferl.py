@@ -258,7 +258,7 @@ def slab_row_index(num_envs, horizon, num_minibatches, bptt_horizon):
 # the fused tcgen05 minibatch-update kernel (csrc/mlp_update.cu) is the default where it applies; config.fused_update
 # overrides
 FUSED_UPDATE_DEFAULT = True
-FUSED_UPDATE_DW_DEFAULT = 'kernel'      # dW_enc inside the fused kernel (6.45 ms/step at C2) vs 'cublas' (dPre to HBM + split-K GEMM, 7.7 ms)
+FUSED_UPDATE_DW_DEFAULT = 'kernel'      # the fused kernel forms dW_enc itself (the only mode); bench.py reads this name
 # the persistent rollout kernel (pb_rollout_breakout_mlp) likewise; config.fused_rollout overrides
 FUSED_ROLLOUT_DEFAULT = True
 
@@ -332,7 +332,7 @@ class _DefaultMLPUpdate:
                                                  st['step'].data_ptr(), g.data_ptr(), p.numel())
         self._keep = (params, grads)
         self._state_ptrs = self._current_state_ptrs()
-        self.fused_ws, self.used_fused, self.fused_dpre, self.part = None, False, None, None
+        self.fused_ws, self.used_fused, self.part = None, False, None
         self.rows = 0
         self.stats = None
         self.world = torch.distributed.get_world_size() if (torch.distributed.is_available() and
@@ -414,11 +414,6 @@ class _DefaultMLPUpdate:
                 self.fused_ws = torch.empty(lib.pb_mlp_update_workspace_bytes(), dtype=torch.uint8, device=self.gflat.device)
             self.mb_rows = g_ * r_
             m_ = self.model
-            # where dW_enc = dPre^T x is formed: inside the kernel (MN-major UMMAs, dPre never leaves the SM), or by a
-            # library GEMM on dPre written to HBM (config.fused_update_dw = 'cublas')
-            in_kernel = str(getattr(config, 'fused_update_dw', FUSED_UPDATE_DW_DEFAULT)) == 'kernel'
-            if not in_kernel and (self.fused_dpre is None or self.fused_dpre.shape[0] != g_ * r_):
-                self.fused_dpre = torch.empty(g_ * r_, self.hid, dtype=torch.float32, device=self.gflat.device)
             _native.check(lib.pb_mlp_update_fused(
                 _native.ptr(x), x.stride(1), r_, (x.stride(0) // x.stride(1)) if g_ > 1 else r_, g_,
                 _native.ptr(m_.encoder.weight), _native.ptr(m_.encoder.bias), _native.ptr(self.w_cat), _native.ptr(self.b_cat),
@@ -428,19 +423,7 @@ class _DefaultMLPUpdate:
                 self.n_act, C.c_float(config.clip_coef),
                 int(bool(config.clip_vloss)), C.c_float(config.vf_clip_coef), C.c_float(config.vf_coef),
                 C.c_float(config.ent_coef), _native.ptr(self.gflat), C.c_void_p(self.stats.data_ptr() + 64 * k),
-                _native.ptr(self.fused_ws), self.fused_ws.numel(), None if in_kernel else _native.ptr(self.fused_dpre),
-                None, None, None, _native.stream_ptr()))
-            if not in_kernel:       # split-K batched GEMM per slab + one sum, as in the kernel chain below
-                f_ = x.shape[2]
-                sp = max(1, 64 // g_)
-                while r_ % sp:
-                    sp //= 2
-                if self.part is None or self.part.shape != (g_ * sp, self.hid, f_):
-                    self.part = torch.empty(g_ * sp, self.hid, f_, dtype=torch.float32, device=x.device)
-                for g in range(g_):
-                    torch.bmm(self.fused_dpre[g * r_:(g + 1) * r_].view(sp, r_ // sp, self.hid).transpose(1, 2),
-                              x[g].view(sp, r_ // sp, f_), out=self.part[g * sp:(g + 1) * sp])
-                torch.sum(self.part, 0, out=self.dw_enc)
+                _native.ptr(self.fused_ws), self.fused_ws.numel(), None, None, None, None, _native.stream_ptr()))
             self.used_fused = True
             return
         x = x.float()
@@ -487,8 +470,7 @@ class _DefaultMLPUpdate:
         lib = _native.lib()
         hyper = (C.c_float(float(config.max_grad_norm)), C.c_float(1.0 / self.world),
                  C.c_float(0.0 if lr_dev is not None else float(lr)), lr_dev, C.c_float(b1), C.c_float(b2), C.c_float(g['eps']), None)
-        in_kernel = str(getattr(config, 'fused_update_dw', FUSED_UPDATE_DW_DEFAULT)) == 'kernel'
-        if self.used_fused and in_kernel and (self.world == 1 or self.peer is not None) and bool(getattr(config, 'adam_parts', True)):
+        if self.used_fused and (self.world == 1 or self.peer is not None):
             # the fused update's reduce step left the gradient's sum of squares as partial sums: multi-CTA clip + Adam without a
             # norm pass; several ranks: sliced peer all-reduce first, which leaves its own partial sums of squares
             m = self.model

@@ -1,8 +1,8 @@
 // mlp_update.cu -- the whole minibatch forward + PPO loss + backward of models.Default in ONE persistent
 // tcgen05 kernel: the observations are read from HBM once, `hidden` / `dPre` never leave the SM.
 //
-// Replaces, per minibatch of clean_pufferl.train (/root/reference/clean_pufferl.py:186-244; policy =
-// /root/reference/pufferlib/models.py:12-62 with 128 input features, 128 hidden units, <= 7 actions), the chain
+// Replaces, per minibatch of clean_pufferl.train (the reference's clean_pufferl.py:186-244; policy = its
+// pufferlib/models.py:12-62 with 128 input features, 128 hidden units, <= 7 actions), the chain
 //     hidden = relu(x W_enc^T + b_enc)            (cuBLAS GEMM, writes 268 MB at M = 524288)
 //     out    = hidden W_heads^T + b_heads         (cuBLAS GEMM, reads hidden)
 //     pb_ppo_loss(out) -> dOut, statistics        (csrc/ppo_loss.cu)
@@ -11,17 +11,25 @@
 // which streams `hidden` / `dPre` through HBM five times (1.9 GB, ~350 us per minibatch).  Here the algorithmic traffic is
 // x once (268 MB) + 28 B of per-row scalars (ncu: 287 MB of DRAM traffic per launch).
 //
-// Two kernels, the second one is the product path (pb_mlp_update_set_variant, default 2; DESIGN.md 3b):
-//   k_mlp_update_fused (variant 1, and the dPre-to-HBM mode of both variants): every x tile is loaded twice, K-major for
-//       the forward product and MN-major (SWIZZLE_128B_BASE32B, the only MN-major layout the tensor core takes for 32-bit
-//       operands) for dW_enc^T = x^T dPre; thread-per-row epilogue with the head products as constant-bank FFMAs.  293 us.
-//   k_mlp_update_xt (variant 2): ONE x layout; x^T is formed on the tensor core by a "sliding identity" MMA into tensor
-//       memory and enters the dW product as a TS operand; the 64 KB that frees hold a whole tile of dPre; 16 epilogue warps
-//       do all per-element products on mma.sync fragments.  168-190 us.
-// Both: warp 0 TMA producer, warp 1 single-thread tcgen05.mma issue + TMEM allocation, the rest epilogue; the dW_enc^T
-// accumulator lives in TMEM across all tiles of a CTA; per-CTA partials go to a workspace and k_update_reduce sums them
-// deterministically into the flat gradient buffer [dW_enc (hid x feat) | dW_heads (8 x hid) | db_enc | db_heads] of
-// clean_pufferl._DefaultMLPUpdate, leaving per-block sums of squares for pb_clip_adam_parts.
+// k_mlp_update_xt (DESIGN.md 3b): warp 0 TMA producer, warp 1 single-thread tcgen05.mma issue + TMEM allocation, warps
+// 2..17 epilogue.  Every x tile is loaded ONCE, K-major SWIZZLE_128B, and feeds three tensor-core products:
+//     h[row][hid]       = x . W_enc^T       SS MMA, two accumulator stages in tensor memory
+//     x^T[feat][row]    = I . x^T           SS MMA: A = an 8 KB "sliding identity" (no-swizzle K-major), B = the same x tile
+//     dW^T[feat][hid]  += x^T . dPre        TS MMA: A = that accumulator (lanes = feat, columns = rows), B = dPre written by the
+//                                           epilogue as K-major SWIZZLE_128B blocks [128 hid][32 rows] (one per row quadrant)
+// The dW product contracts over rows, so x has to enter it transposed.  The tensor core takes transposed (MN-major) 32-bit
+// operands from shared memory only in the SWIZZLE_128B_BASE32B layout, which would mean a second load of every tile in a
+// second layout.  Instead the second product writes x^T into tensor memory, where a TS MMA reads it as its A operand.  It
+// is exact (every product is with 1.0 or 0.0) and runs on a tensor pipe with slack (validated on hardware by
+// tests/experimental/check_umma_transpose.py).  The identity is one 8x8 block at core matrix 15 of a 32-matrix strip of
+// zeros; MMA k starts (15 - k) core matrices into the strip, so row group k of A sees the identity and every other row
+// group zeros: one 8 KB buffer serves all 16 K-steps.  The shared memory a second x tile would take holds a whole tile of
+// dPre instead, so the epilogue never waits for the tensor core inside a tile, and there is room for 16 epilogue warps
+// (4 per scheduler: row quadrant q x column quarter c) that do all per-element products on mma.sync fragments.
+// TMEM: [0,256) two forward accumulators, [256,384) x^T, [384,512) dW^T.  The dW_enc^T accumulator lives across all
+// tiles of a CTA; per-CTA partials go to a workspace and k_update_reduce sums them deterministically into the flat
+// gradient buffer [dW_enc (hid x feat) | dW_heads (8 x hid) | db_enc | db_heads] of clean_pufferl._DefaultMLPUpdate,
+// leaving per-block sums of squares for pb_clip_adam_parts.
 //
 // Descriptor encodings were validated on hardware with csrc/experimental/umma_probe.cu (tests/experimental/
 // check_umma_probe.py, check_umma_transpose.py).  Every mbarrier wait is bounded (tma.cuh: __trap instead of a hang).
@@ -37,25 +45,8 @@ constexpr int TILE_M = 128, HID = 128, FEAT = 128, NO = 8;
 constexpr int KBLK = 32;                               // floats per 128-byte swizzle row
 constexpr int KBLK_BYTES = TILE_M * KBLK * 4;          // 16 KiB: one [128 rows][32 floats] box
 constexpr int TILE_BYTES = 4 * KBLK_BYTES;             // 64 KiB
-constexpr int NCHUNK = 4, CHUNK_COLS = 32;
-constexpr int CHUNK_BYTES = TILE_M * CHUNK_COLS * 4;   // 16 KiB: [128 rows][32 hid] MN-major (N contiguous)
-constexpr int SMEM_W = 0;                              // W_enc, K-major SWIZZLE_128B, resident
-constexpr int SMEM_XK = TILE_BYTES;                    // x tile for the forward product: K-major SWIZZLE_128B
-constexpr int SMEM_XM = 2 * TILE_BYTES;                // x tile for the dW product: MN-major SWIZZLE_128B_BASE32B
-constexpr int SMEM_CH = 3 * TILE_BYTES;                // two dPre chunk buffers (one per column half)
-constexpr int SMEM_BAR = SMEM_CH + 2 * CHUNK_BYTES;
-constexpr int SMEM_TOTAL = SMEM_BAR + 256;
-constexpr int THREADS = 320;                           // warp 0 TMA, warp 1 MMA, warps 2..9 epilogue
 constexpr int TMEM_COLS = 512;
-constexpr int TMEM_DW = 256;                           // first column of the dW^T accumulator
-constexpr int TMEM_XCHG = 384;                         // 16 columns: the partial head sums the two warps of a row exchange
 constexpr int TAIL = NO * HID + HID + NO;              // dW_heads | db_enc | db_heads
-static_assert(SMEM_TOTAL <= 232448, "shared memory budget");
-
-// W_heads [8][128], b_enc [128], b_heads [8]: uniform per warp at every use -> constant-bank operands of the FFMAs
-__constant__ float c_wh[NO * HID];
-__constant__ float c_benc[HID];
-__constant__ float c_bh[NO];
 
 struct FusedParams {
     const int64_t* actions;
@@ -75,14 +66,13 @@ struct FusedParams {
     float* part_dw;            // [grid][FEAT][HID]
     float* part_tail;          // [grid][TAIL]
     double* stats;             // [8]
-    float* dpre_out;           // DW_KERNEL = false: dPre [m][128] (slab-major rows) for the caller's dW GEMM
     float* dbg_hidden;         // nullable [m][128]
     float* dbg_dpre;           // nullable [m][128]
     float* dbg_dout;           // nullable [m][8]
-    const float* w_heads;      // [8][128], b_enc [128], b_heads [8] in global memory (variant 2 reads them directly)
+    const float* w_heads;      // [8][128], b_enc [128], b_heads [8] in global memory
     const float* b_enc;
     const float* b_heads;
-    long long* dbg_clk;        // profiling only: [grid][18 warps][4 tiles][8 events] SM clock stamps of tiles 8..11 (variant 2)
+    long long* dbg_clk;        // profiling only: [grid][18 warps][4 tiles][8 events] SM clock stamps of tiles 8..11
 };
 
 __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
@@ -95,21 +85,14 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// SWIZZLE_128B descriptors (PTX ISA tcgen05 shared-memory descriptor; cute/arch/mma_sm100_desc.hpp): start>>4 | LBO>>4 <<16
-// | SBO>>4 <<32 | version 1 <<46 | layout 2 <<61.  K-major: LBO unused (1), SBO = 1024 B between 8-row groups.
-// MN-major: LBO = distance between 32-element MN groups, SBO = 1024 B between 8-k groups.
+// K-major SWIZZLE_128B descriptor (PTX ISA tcgen05 shared-memory descriptor; cute/arch/mma_sm100_desc.hpp): start>>4 |
+// LBO>>4 <<16 | SBO>>4 <<32 | version 1 <<46 | layout 2 <<61, with LBO unused (1) and SBO = 1024 B between 8-row groups.
 __device__ __forceinline__ uint64_t desc_kmajor(uint32_t saddr) {
     return (uint64_t)((saddr & 0x3FFFF) >> 4) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
 }
-// MN-major 32-bit operands: layout type 1 (SWIZZLE_128B_BASE32B), atoms of 4 k x 128 B, SBO = 512 B between 4-k groups,
-// LBO = distance between 32-element MN groups
-__device__ __forceinline__ uint64_t desc_mn32(uint32_t saddr, uint32_t lbo_bytes) {
-    return (uint64_t)((saddr & 0x3FFFF) >> 4) | ((uint64_t)(lbo_bytes >> 4) << 16) | (32ull << 32) | (1ull << 46) | (1ull << 61);
-}
-// instruction descriptor: D fmt F32 (1<<4) | A TF32 (2<<7) | B TF32 (2<<10) | A major bit 15 | B major bit 16 | N>>3 <<17 | M>>4 <<24
+// instruction descriptor: D fmt F32 (1<<4) | A TF32 (2<<7) | B TF32 (2<<10) | both K-major (bits 15, 16 clear) | N>>3 <<17 |
+// M>>4 <<24.  Used by all three products (M = N = 128).
 constexpr uint32_t IDESC_FWD = (1u << 4) | (2u << 7) | (2u << 10) | ((HID >> 3) << 17) | ((TILE_M >> 4) << 24);
-constexpr uint32_t IDESC_DW = (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((CHUNK_COLS >> 3) << 17) |
-                              ((FEAT >> 4) << 24);
 
 __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
     asm volatile(
@@ -130,22 +113,6 @@ __device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, u
         "}\n" ::"r"(tmem_d),
         "r"(tmem_a), "l"(b_desc), "r"(idesc), "r"(acc)
         : "memory");
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const float (&r)[8]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr),
-                 "r"(__float_as_uint(r[0])), "r"(__float_as_uint(r[1])), "r"(__float_as_uint(r[2])), "r"(__float_as_uint(r[3])),
-                 "r"(__float_as_uint(r[4])), "r"(__float_as_uint(r[5])), "r"(__float_as_uint(r[6])), "r"(__float_as_uint(r[7]))
-                 : "memory");
-}
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&r)[8]) {
-    uint32_t u[8];
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7])
-                 : "r"(taddr)
-                 : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 8; ++i) r[i] = __uint_as_float(u[i]);
 }
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -176,480 +143,12 @@ __device__ __forceinline__ uint32_t to_tf32(float x) {
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
     return r;
 }
-__device__ __forceinline__ void mma_tf32(float& c0, float& c1, float& z0, float& z1, const uint32_t (&a)[2], uint32_t b0,
-                                         uint32_t b1) {
-    // m16n8k8: rows 8..15 of A are zero (a1 = a3 = 0), their accumulators (z0, z1) are shared dummies
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(c0), "+f"(c1), "+f"(z0), "+f"(z1)
-                 : "r"(a[0]), "r"(0u), "r"(a[1]), "r"(0u), "r"(b0), "r"(b1));
-}
 
-// The row math of k_ppo_loss<PACKED> (csrc/ppo_loss.cu; clean_pufferl.py:202-238 + frameworks/cleanrl.py:25-47):
-// z[0..n_act) logits, z[n_act] value -> dOut[8] (already scaled by 1/M) and the six per-row statistics.
+// The row math of k_ppo_loss (csrc/ppo_loss.cu, the statement of the math; clean_pufferl.py:202-238 +
+// frameworks/cleanrl.py:25-47) with FOUR lanes per row: lane `sub` (0..3) of the row owns outputs sub and sub + 4 (logits
+// below n_act, the value at index n_act); row-wide maxima / sums go through width-4 shuffles.  Every lane of the warp must
+// call it (shuffles).  Returns dOut of the two owned outputs (already scaled by 1/M) and the six per-row statistics.
 struct RowStats { float pg, v, ent, okl, kl, clipped; };
-__device__ __forceinline__ RowStats ppo_row(const float (&zin)[8], const FusedParams& p, int act, float old_lp, float adv,
-                                            float ret, float old_v, float (&gro)[8]) {
-    float z[8];
-    float mx = -INFINITY;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        z[k] = zin[k];
-        if (k < p.n_act) mx = fmaxf(mx, z[k]);
-    }
-    float v_new = 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k)
-        if (k == p.n_act) v_new = z[k];
-    float sum = 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k)
-        if (k < p.n_act) sum += expf(z[k] - mx);
-    const float lse = mx + logf(sum);
-    const int a = act < 0 ? 0 : (act >= p.n_act ? p.n_act - 1 : act);
-    float ent = 0.f, nl_a = 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k)
-        if (k < p.n_act) {
-            const float nl = z[k] - lse, pk = expf(nl);
-            ent -= pk * nl;
-            if (k == a) nl_a = nl;
-            z[k] = nl;
-        }
-    const float logratio = nl_a - old_lp;
-    const float ratio = expf(logratio);
-    const float pg1 = -adv * ratio;
-    const float rc = fminf(fmaxf(ratio, 1.f - p.clip), 1.f + p.clip);
-    const float pg2 = -adv * rc;
-    const float pg = fmaxf(pg1, pg2);
-    const float in_range = (ratio >= 1.f - p.clip && ratio <= 1.f + p.clip) ? 1.f : 0.f;
-    float g_ratio;
-    if (pg1 > pg2) g_ratio = -adv;
-    else if (pg1 < pg2) g_ratio = -adv * in_range;
-    else g_ratio = 0.5f * (-adv) + 0.5f * (-adv * in_range);
-    const float inv_m = 1.0f / (float)p.m;
-    const float g_nlp = g_ratio * ratio * inv_m;
-    const float dv = v_new - ret;
-    float vl, g_v;
-    if (p.clip_vloss) {
-        const float d = v_new - old_v;
-        const float dc = fminf(fmaxf(d, -p.vclip), p.vclip);
-        const float vc = old_v + dc;
-        const float vu = dv * dv, vcl = (vc - ret) * (vc - ret);
-        vl = fmaxf(vu, vcl);
-        const float v_in = (d >= -p.vclip && d <= p.vclip) ? 1.f : 0.f;
-        const float gu = 2.f * dv, gc = 2.f * (vc - ret) * v_in;
-        g_v = vu > vcl ? gu : (vu < vcl ? gc : 0.5f * (gu + gc));
-    } else {
-        vl = dv * dv;
-        g_v = 2.f * dv;
-    }
-    const float gv_out = 0.5f * p.vf_coef * g_v * inv_m;
-    const float g_ent = p.ent_coef * inv_m;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        gro[k] = 0.f;
-        if (k < p.n_act) {
-            const float pk = expf(z[k]);
-            gro[k] = g_nlp * ((k == a ? 1.f : 0.f) - pk) + g_ent * pk * (z[k] + ent);
-        }
-        if (k == p.n_act) gro[k] = gv_out;
-    }
-    RowStats s;
-    s.pg = pg; s.v = vl; s.ent = ent; s.okl = -logratio; s.kl = (ratio - 1.f) - logratio;
-    s.clipped = fabsf(ratio - 1.f) > p.clip ? 1.f : 0.f;
-    return s;
-}
-
-// NH = live rows of the 8-row head matrix (n_act logits + the value): rows >= NH are zero padding, their products are skipped
-// byte offset of element (row r, column j) of a [128 rows][32 floats] chunk in the SWIZZLE_128B_BASE32B layout (32-byte
-// pieces of a 128-byte row, piece index ^= row & 3): the layout the tensor core requires for MN-major 32-bit operands
-// (UMMA layout type 1; TMA writes it with CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B).  Conflict-free for the fragment loads of
-// the dW_heads mma.sync and for the column sums; 2-way for the row-owner 128-bit stores.
-__device__ __forceinline__ uint32_t chunk32_off(int r, int j) {
-    return (uint32_t)(r * 128 + ((((j >> 3) ^ (r & 3))) << 5) + ((j & 7) << 2));
-}
-
-// DW_KERNEL = true : dW_enc^T accumulated in TMEM by MN-major UMMAs (x tile loaded a second time in the BASE32B layout)
-// DW_KERNEL = false: dPre goes to HBM (p.dpre_out) and the caller forms dW_enc = dPre^T x with a library GEMM
-template <int NH, bool DW_KERNEL>
-__global__ void __launch_bounds__(THREADS, 1)
-k_mlp_update_fused(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_x32,
-                   const __grid_constant__ CUtensorMap map_w, const FusedParams p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + SMEM_BAR);
-    uint64_t* w_full = bars;              // W_enc resident
-    uint64_t* xk_full = bars + 1;         // forward operand tile (K-major SW128) landed
-    uint64_t* xk_empty = bars + 2;        // ... consumed by the forward MMAs
-    uint64_t* xm_full = bars + 3;         // dW operand tile (MN-major BASE32B) landed
-    uint64_t* xm_empty = bars + 4;        // ... consumed by the dW MMAs of the tile
-    uint64_t* h_full = bars + 5;          // [2] forward accumulator complete
-    uint64_t* h_empty = bars + 7;         // [2] drained by the 8 epilogue warps
-    uint64_t* dp_full = bars + 9;         // [2] dPre chunk of column half hh written (4 warps)
-    uint64_t* dp_empty = bars + 11;       // [2] ... consumed by its dW MMAs
-    uint64_t* dw_done = bars + 13;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 14);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        mbar_init(w_full, 1);
-        mbar_init(xk_full, 1);
-        mbar_init(xk_empty, 1);
-        mbar_init(xm_full, 1);
-        mbar_init(xm_empty, 1);
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&h_full[i], 1);
-            mbar_init(&h_empty[i], 8);
-            mbar_init(&dp_full[i], 4);
-            mbar_init(&dp_empty[i], 1);
-        }
-        mbar_init(dw_done, 1);
-        mbar_fence_init();
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                     "r"((uint32_t)TMEM_COLS)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const int n_my = (p.n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // tiles of this CTA (>= 1)
-
-    // per-thread results of the epilogue warps, reduced after the role loops.  Epilogue warp (q, hh): TMEM lane quadrant q
-    // (tile rows 32q..32q+31), column half hh = hidden units 64hh..64hh+63 = chunks 2hh, 2hh+1.
-    float acc_wh[2][4][2];               // dW_heads[a = lane>>2][j = 32(2hh+cc) + 8nb + 2(lane&3) + {0,1}]  (this warp's rows)
-    float acc_benc[2];                   // db_enc[32(2hh+cc) + lane]
-    float acc_bh[NO];                    // db_heads (this thread's rows; hh == 0 only)
-    double st[6] = {0, 0, 0, 0, 0, 0};
-#pragma unroll
-    for (int cc = 0; cc < 2; ++cc) {
-        acc_benc[cc] = 0.f;
-#pragma unroll
-        for (int nb = 0; nb < 4; ++nb) acc_wh[cc][nb][0] = acc_wh[cc][nb][1] = 0.f;
-    }
-#pragma unroll
-    for (int k = 0; k < NO; ++k) acc_bh[k] = 0.f;
-
-    if (warp == 0) {
-        // ================= TMA producer =================
-        if (lane == 0) {
-            mbar_expect_tx(w_full, TILE_BYTES);
-            for (int kb = 0; kb < 4; ++kb) tma_load_2d(smem + SMEM_W + kb * KBLK_BYTES, &map_w, kb * KBLK, 0, w_full);
-            for (int it = 0; it < n_my; ++it) {
-                const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-                const int64_t row0 = (int64_t)(tile / p.tiles_per_slab) * p.slab_stride_rows +
-                                     (int64_t)(tile % p.tiles_per_slab) * TILE_M;
-                mbar_wait(xk_empty, (uint32_t)((it & 1) ^ 1));          // forward MMAs of tile it-1 have read the buffer
-                mbar_expect_tx(xk_full, TILE_BYTES);
-                for (int kb = 0; kb < 4; ++kb) tma_load_2d(smem + SMEM_XK + kb * KBLK_BYTES, &map_x, kb * KBLK, (int)row0, xk_full);
-                if (DW_KERNEL) {   // the same rows again (L2 hits) in the MN-major layout of the dW product
-                    mbar_wait(xm_empty, (uint32_t)((it & 1) ^ 1));      // dW MMAs of tile it-1 done
-                    mbar_expect_tx(xm_full, TILE_BYTES);
-                    for (int kb = 0; kb < 4; ++kb)
-                        tma_load_2d(smem + SMEM_XM + kb * KBLK_BYTES, &map_x32, kb * KBLK, (int)row0, xm_full);
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ================= MMA issuer (one thread) =================
-        if (lane == 0) {
-            const uint32_t w_addr = smem_u32(smem + SMEM_W);
-            const uint32_t xk_addr = smem_u32(smem + SMEM_XK), xm_addr = smem_u32(smem + SMEM_XM);
-            auto forward = [&](int it) {
-                const int s = it & 1, ph = (it >> 1) & 1;
-                mbar_wait(&h_empty[s], ph ^ 1);                  // epilogue drained accumulator stage s (tile it - 2)
-                mbar_wait(xk_full, (uint32_t)(it & 1));          // x tile landed
-                tc_fence_after();
-                const uint32_t d_tmem = tmem_base + (uint32_t)(s * HID);
-#pragma unroll
-                for (int kb = 0; kb < 4; ++kb)
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-                        umma_tf32(d_tmem, desc_kmajor(xk_addr + kb * KBLK_BYTES + k * 32),
-                                  desc_kmajor(w_addr + kb * KBLK_BYTES + k * 32), IDESC_FWD, (kb | k) ? 1u : 0u);
-                umma_commit(&h_full[s]);
-                umma_commit(xk_empty);                           // the K-major tile may be overwritten: next tile's load starts
-            };
-            mbar_wait(w_full, 0);
-            forward(0);
-            for (int it = 0; it < n_my; ++it) {
-                if (it + 1 < n_my) forward(it + 1);              // overlaps the epilogue of tile `it`
-                if (DW_KERNEL) {
-                    mbar_wait(xm_full, (uint32_t)(it & 1));
-                    // chunks arrive alternately from the two column halves: 0 (hh 0), 2 (hh 1), 1 (hh 0), 3 (hh 1)
-#pragma unroll 1
-                    for (int i = 0; i < NCHUNK; ++i) {
-                        const int hh = i & 1, cc = i >> 1, c = 2 * hh + cc;
-                        const int u = it * 2 + cc;               // use count of chunk buffer hh
-                        mbar_wait(&dp_full[hh], (uint32_t)(u & 1));
-                        tc_fence_after();
-                        const uint32_t ch_addr = smem_u32(smem + SMEM_CH + hh * CHUNK_BYTES);
-                        const uint32_t d_tmem = tmem_base + (uint32_t)(TMEM_DW + c * CHUNK_COLS);
-#pragma unroll
-                        for (int k = 0; k < TILE_M / 8; ++k)      // K = 8 rows per MMA = two 512-byte atoms
-                            umma_tf32(d_tmem, desc_mn32(xm_addr + k * 1024, KBLK_BYTES), desc_mn32(ch_addr + k * 1024, KBLK_BYTES),
-                                      IDESC_DW, (it | k) ? 1u : 0u);
-                        umma_commit(&dp_empty[hh]);
-                    }
-                    umma_commit(xm_empty);
-                }
-            }
-            umma_commit(dw_done);
-        }
-    } else {
-        // ================= epilogue warps: thread = tile row (TMEM lane 32q + lane), column half hh =================
-        const int q = warp & 3, hh = (warp - 2) >> 2;
-        const int g = lane >> 2, t = lane & 3;
-        const int rloc = 32 * q + lane;                        // row inside the tile
-        uint8_t* buf = smem + SMEM_CH + hh * CHUNK_BYTES;      // this half's chunk buffer; this warp owns rows 32q..32q+31
-        const uint32_t xchg = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)TMEM_XCHG;
-        float z0 = 0.f, z1 = 0.f;                              // dummy accumulators of the zero A rows
-        for (int it = 0; it < n_my; ++it) {
-            const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-            const int s = it & 1, ph = (it >> 1) & 1;
-            const int slab = tile / p.tiles_per_slab;
-            const int64_t lrow = (int64_t)(tile % p.tiles_per_slab) * TILE_M + rloc;
-            const bool valid = lrow < p.slab_rows;
-            const int64_t i = (int64_t)slab * p.slab_rows + lrow;            // slab-major position (dPre / debug rows)
-            const int64_t ri = (int64_t)slab * p.row_slab_stride + lrow;     // position in the per-row arrays
-            int act = 0;
-            float old_lp = 0.f, adv = 0.f, ret = 0.f, old_v = 0.f;
-            if (valid) {
-                act = (int)p.actions[ri];
-                old_lp = p.old_logprobs[ri];
-                adv = p.adv[ri];
-                old_v = (p.clip_vloss || !p.returns) ? p.old_values[ri] : 0.f;
-                ret = p.returns ? p.returns[ri] : adv + old_v;
-                if (p.adv_norm) adv = (adv - p.adv_norm[0]) * p.adv_norm[1];
-            }
-            mbar_wait(&h_full[s], ph);
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(s * HID);
-
-            // ---- pass 1: this half's share of the head products, exchanged with the partner warp through tensor memory
-            float out[NO];
-#pragma unroll
-            for (int a = 0; a < NO; ++a) out[a] = 0.f;
-#pragma unroll
-            for (int cc = 0; cc < 2; ++cc) {
-                float v[32];
-                if (hh == 0) {      // (compile-time column offsets: every c_wh / c_benc operand is a constant-bank immediate)
-                    tmem_ld32(taddr + 32 * cc, v);
-#pragma unroll
-                    for (int k = 0; k < 32; ++k) {
-                        const float rh = fmaxf(v[k] + c_benc[32 * cc + k], 0.f);
-#pragma unroll
-                        for (int a = 0; a < NH; ++a) out[a] = fmaf(rh, c_wh[a * HID + 32 * cc + k], out[a]);
-                    }
-                } else {
-                    tmem_ld32(taddr + 64 + 32 * cc, v);
-#pragma unroll
-                    for (int k = 0; k < 32; ++k) {
-                        const float rh = fmaxf(v[k] + c_benc[64 + 32 * cc + k], 0.f);
-#pragma unroll
-                        for (int a = 0; a < NH; ++a) out[a] = fmaf(rh, c_wh[a * HID + 64 + 32 * cc + k], out[a]);
-                    }
-                }
-            }
-            {
-            tmem_st8(xchg + 8 * hh, out);
-            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-            tc_fence_before();
-            asm volatile("bar.sync %0, 64;" ::"r"(1 + q) : "memory");     // the two warps of quadrant q
-            tc_fence_after();
-            }
-            {
-                float other[NO];
-                tmem_ld8(xchg + 8 * (hh ^ 1), other);
-#pragma unroll
-                for (int a = 0; a < NO; ++a) out[a] = (hh == 0 ? out[a] + other[a] : other[a] + out[a]) + c_bh[a];   // same order in both
-            }
-            // the partner must have read my partial before the next tile overwrites it: second rendezvous at the end of the tile
-
-            // ---- loss row math -> dOut (both warps of the pair compute it; the statistics are taken by hh == 0)
-            float dO[NO];
-#pragma unroll
-            for (int a = 0; a < NO; ++a) dO[a] = 0.f;
-            if (valid) {
-                const RowStats rs = ppo_row(out, p, act, old_lp, adv, ret, old_v, dO);
-                if (hh == 0) {
-                    st[0] += rs.pg; st[1] += rs.v; st[2] += rs.ent; st[3] += rs.okl; st[4] += rs.kl; st[5] += rs.clipped;
-                    if (p.dbg_dout) {
-                        *reinterpret_cast<float4*>(p.dbg_dout + i * 8) = make_float4(dO[0], dO[1], dO[2], dO[3]);
-                        *reinterpret_cast<float4*>(p.dbg_dout + i * 8 + 4) = make_float4(dO[4], dO[5], dO[6], dO[7]);
-                    }
-                }
-            }
-            if (hh == 0) {
-#pragma unroll
-                for (int a = 0; a < NO; ++a) acc_bh[a] += dO[a];
-            }
-
-            // ---- A fragments of the dW_heads mma (A[m = head a][k = row]) staged through this warp's rows of its half's
-            //      chunk buffer (32 B per row; private to the warp until a dPre chunk is published)
-            uint32_t afr[4][2];
-            {
-                if (DW_KERNEL) mbar_wait(&dp_empty[hh], (uint32_t)(((it * 2) & 1) ^ 1));
-                *reinterpret_cast<float4*>(buf + rloc * 128) = make_float4(dO[0], dO[1], dO[2], dO[3]);
-                *reinterpret_cast<float4*>(buf + rloc * 128 + 16) = make_float4(dO[4], dO[5], dO[6], dO[7]);
-                __syncwarp();
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {
-                    afr[ks][0] = to_tf32(*reinterpret_cast<const float*>(buf + (32 * q + 8 * ks + t) * 128 + g * 4));
-                    afr[ks][1] = to_tf32(*reinterpret_cast<const float*>(buf + (32 * q + 8 * ks + t + 4) * 128 + g * 4));
-                }
-                __syncwarp();
-            }
-
-            // ---- pass 2: this half's two 32-column chunks: dPre, dW_heads, db_enc
-#pragma unroll
-            for (int cc = 0; cc < 2; ++cc) {
-                float v[32], dp[32];
-                const int col0 = 64 * hh + 32 * cc;           // first hidden unit of the chunk (hh is warp-uniform)
-                tmem_ld32(taddr + col0, v);
-                if (hh == 0) {
-#pragma unroll
-                    for (int k = 0; k < 32; ++k) {
-                        const float pre = v[k] + c_benc[32 * cc + k];
-                        float gk = 0.f;
-#pragma unroll
-                        for (int a = 0; a < NH; ++a) gk = fmaf(dO[a], c_wh[a * HID + 32 * cc + k], gk);
-                        dp[k] = pre > 0.f ? gk : 0.f;
-                        v[k] = fmaxf(pre, 0.f);
-                    }
-                } else {
-#pragma unroll
-                    for (int k = 0; k < 32; ++k) {
-                        const float pre = v[k] + c_benc[64 + 32 * cc + k];
-                        float gk = 0.f;
-#pragma unroll
-                        for (int a = 0; a < NH; ++a) gk = fmaf(dO[a], c_wh[a * HID + 64 + 32 * cc + k], gk);
-                        dp[k] = pre > 0.f ? gk : 0.f;
-                        v[k] = fmaxf(pre, 0.f);
-                    }
-                }
-                if (valid && p.dbg_hidden) {
-#pragma unroll
-                    for (int k = 0; k < 32; k += 4) {
-                        *reinterpret_cast<float4*>(p.dbg_hidden + i * HID + col0 + k) = make_float4(v[k], v[k + 1], v[k + 2], v[k + 3]);
-                        *reinterpret_cast<float4*>(p.dbg_dpre + i * HID + col0 + k) = make_float4(dp[k], dp[k + 1], dp[k + 2], dp[k + 3]);
-                    }
-                }
-                if (!DW_KERNEL && valid) {    // dPre row segment to HBM (128 contiguous bytes per thread)
-#pragma unroll
-                    for (int k = 0; k < 32; k += 4)
-                        __stcs(reinterpret_cast<float4*>(p.dpre_out + i * HID + col0 + k), make_float4(dp[k], dp[k + 1], dp[k + 2], dp[k + 3]));
-                }
-                if (DW_KERNEL) mbar_wait(&dp_empty[hh], (uint32_t)(((it * 2 + cc) & 1) ^ 1));   // last use of the buffer consumed
-                // relu(h) chunk of this warp's 32 rows (TF32-rounded) -> B fragments of the dW_heads mma
-                {
-#pragma unroll
-                for (int j8 = 0; j8 < 4; ++j8) {
-                    uint8_t* dst = buf + rloc * 128 + ((j8 ^ (rloc & 3)) << 5);
-                    *reinterpret_cast<uint4*>(dst) = make_uint4(to_tf32(v[8 * j8]), to_tf32(v[8 * j8 + 1]), to_tf32(v[8 * j8 + 2]), to_tf32(v[8 * j8 + 3]));
-                    *reinterpret_cast<uint4*>(dst + 16) = make_uint4(to_tf32(v[8 * j8 + 4]), to_tf32(v[8 * j8 + 5]), to_tf32(v[8 * j8 + 6]), to_tf32(v[8 * j8 + 7]));
-                }
-                __syncwarp();
-#pragma unroll
-                for (int ks = 0; ks < 4; ++ks) {
-                    const int r0 = 32 * q + 8 * ks + t;
-#pragma unroll
-                    for (int nb = 0; nb < 4; ++nb) {
-                        const uint32_t b0 = *reinterpret_cast<const uint32_t*>(buf + chunk32_off(r0, 8 * nb + g));
-                        const uint32_t b1 = *reinterpret_cast<const uint32_t*>(buf + chunk32_off(r0 + 4, 8 * nb + g));
-                        mma_tf32(acc_wh[cc][nb][0], acc_wh[cc][nb][1], z0, z1, afr[ks], b0, b1);
-                    }
-                }
-                __syncwarp();
-                }
-                // dPre chunk -> the same rows, BASE32B layout (the MN-major B operand of the dW UMMA)
-#pragma unroll
-                for (int j8 = 0; j8 < 4; ++j8) {
-                    uint8_t* dst = buf + rloc * 128 + ((j8 ^ (rloc & 3)) << 5);
-                    *reinterpret_cast<float4*>(dst) = make_float4(dp[8 * j8], dp[8 * j8 + 1], dp[8 * j8 + 2], dp[8 * j8 + 3]);
-                    *reinterpret_cast<float4*>(dst + 16) = make_float4(dp[8 * j8 + 4], dp[8 * j8 + 5], dp[8 * j8 + 6], dp[8 * j8 + 7]);
-                }
-                if (DW_KERNEL) fence_proxy_async_smem();
-                __syncwarp();
-                if (DW_KERNEL && lane == 0) mbar_arrive(&dp_full[hh]);
-                // db_enc: column sums over this warp's rows (the UMMA only reads the buffer)
-                float cs = 0.f;
-#pragma unroll 8
-                for (int r = 0; r < 32; ++r) cs += *reinterpret_cast<const float*>(buf + chunk32_off(32 * q + r, lane));
-                acc_benc[cc] += cs;
-                __syncwarp();                                    // (mode without UMMA: the next chunk overwrites the rows)
-            }
-            tc_fence_before();
-            asm volatile("bar.sync %0, 64;" ::"r"(1 + q) : "memory");     // both warps are done with the exchange columns
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&h_empty[s]);
-        }
-        // ---- the dW^T accumulator of this CTA: TMEM lane = feature, column = hidden unit; this warp dumps its column half
-        if (DW_KERNEL) {
-            mbar_wait(dw_done, 0);
-            tc_fence_after();
-            float* pd = p.part_dw + ((int64_t)blockIdx.x * FEAT + rloc) * HID;
-#pragma unroll 1
-            for (int cc = 0; cc < 2; ++cc) {
-                float v[32];
-                const int col0 = 64 * hh + 32 * cc;
-                tmem_ld32(tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(TMEM_DW + col0), v);
-#pragma unroll
-                for (int k = 0; k < 32; k += 4)
-                    *reinterpret_cast<float4*>(pd + col0 + k) = make_float4(v[k], v[k + 1], v[k + 2], v[k + 3]);
-            }
-        }
-        if (hh == 0) {   // loss statistics: warp reduce, one fp64 atomic per warp and statistic
-#pragma unroll
-            for (int k = 0; k < 6; ++k) {
-                double x = st[k];
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) x += __shfl_xor_sync(0xffffffffu, x, off);
-                if (lane == 0) atomicAdd(p.stats + k, x);
-            }
-        }
-    }
-
-    // ================= CTA reduction of the small gradients (8 epilogue warps -> one partial row) =================
-    tc_fence_before();
-    __syncthreads();                       // every role is done: all MMAs retired, all TMA loads consumed
-    float* red = reinterpret_cast<float*>(smem + SMEM_XK);         // [4 quadrants][TAIL] scratch in the (now idle) x tile
-    if (warp >= 2) {
-        const int q = warp & 3, hh = (warp - 2) >> 2, g = lane >> 2, t = lane & 3;
-        float* mine = red + q * TAIL;      // the two warps of a quadrant fill disjoint columns of the same row
-#pragma unroll
-        for (int cc = 0; cc < 2; ++cc) {
-            const int col0 = 64 * hh + 32 * cc;
-#pragma unroll
-            for (int nb = 0; nb < 4; ++nb) {
-                mine[g * HID + col0 + 8 * nb + 2 * t] = acc_wh[cc][nb][0];
-                mine[g * HID + col0 + 8 * nb + 2 * t + 1] = acc_wh[cc][nb][1];
-            }
-            mine[NO * HID + col0 + lane] = acc_benc[cc];
-        }
-        if (hh == 0) {
-#pragma unroll
-            for (int k = 0; k < NO; ++k) {
-                float x = acc_bh[k];
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) x += __shfl_xor_sync(0xffffffffu, x, off);
-                if (lane == 0) mine[NO * HID + HID + k] = x;
-            }
-        }
-    }
-    __syncthreads();
-    float* pt = p.part_tail + (int64_t)blockIdx.x * TAIL;
-    for (int j = threadIdx.x; j < TAIL; j += THREADS) pt[j] = red[j] + red[TAIL + j] + red[2 * TAIL + j] + red[3 * TAIL + j];
-    if (warp == 1)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TMEM_COLS)
-                     : "memory");
-}
-
-// ppo_row with FOUR lanes per row: lane `sub` (0..3) of the row owns outputs sub and sub + 4 (logits below n_act, the value at
-// index n_act); row-wide maxima / sums go through width-4 shuffles.  Same arithmetic as ppo_row, which remains the
-// statement of the math; every lane of the warp must call it (shuffles).  Returns dOut of the two owned outputs.
 __device__ __forceinline__ RowStats ppo_row_sub(float z_lo, float z_hi, int sub, int lane, const FusedParams& p, int act,
                                                 float old_lp, float adv, float ret, float old_v, float& g_lo, float& g_hi) {
     const unsigned full = 0xffffffffu;
@@ -711,18 +210,7 @@ __device__ __forceinline__ RowStats ppo_row_sub(float z_lo, float z_hi, int sub,
     return s;
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// Variant 2: ONE x layout.  The tensor core only takes MN-major 32-bit operands in the BASE32B layout, so variant 1 loads
-// every x tile twice (K-major for the forward product, MN-major for dW) and has no shared memory left to overlap anything.
-// Here the dW product takes x^T from TENSOR memory instead:
-//     x^T[feat][row]    = I . x^T           SS MMA: A = an 8 KB "sliding identity" (no-swizzle K-major, see x2_write_identity),
-//                                           B = the K-major x tile the forward product just read
-//     dW^T[feat][hid]  += x^T . dPre        TS MMA: A = that accumulator (lanes = feat, columns = rows), B = dPre written by the
-//                                           epilogue as K-major SWIZZLE_128B blocks [128 hid][32 rows] (one per row quadrant)
-// (validated on hardware by tests/experimental/check_umma_transpose.py).  The 64 KB the second x tile used to take hold a
-// whole tile of dPre, so the epilogue never waits for the tensor core inside a tile, and there are 16 epilogue warps
-// (4 per scheduler: row quadrant q x column quarter c) instead of 8.
-// TMEM: [0,256) two forward accumulators, [256,384) x^T, [384,512) dW^T (lives across all tiles of the CTA).
+// Shared memory (byte offsets) and tensor memory (columns) of k_mlp_update_xt; the header comment describes the products.
 constexpr int X2_THREADS = 576;                          // warp 0 TMA, warp 1 MMA, warps 2..17 epilogue
 constexpr int X2_W = 0, X2_XK = TILE_BYTES, X2_G = 2 * TILE_BYTES;     // W_enc | x tile | 4 dPre blocks of 16 KiB
 constexpr int X2_XCH = 3 * TILE_BYTES;                   // [4 q][4 c][32 rows][10]: partial head sums (8 used; 10 = bank spread)
@@ -1189,10 +677,6 @@ __global__ void __launch_bounds__(256) k_update_reduce(const float* __restrict__
     const int e = blockIdx.x * 64 + (threadIdx.x & 63), grp = threadIdx.x >> 6;
     constexpr int NDW = FEAT * HID;
     float s = 0.f;
-    if (e < NDW && !part_dw) {                // dW_enc is formed by the caller (dPre went to HBM); whole blocks: NDW % 64 == 0
-        if (threadIdx.x == 0) sumsq_part[blockIdx.x] = 0.0;
-        return;
-    }
     if (e < NDW + TAIL) {
         const float* src = e < NDW ? part_dw + e : part_tail + (e - NDW);
         const int64_t stride = e < NDW ? NDW : TAIL;
@@ -1223,14 +707,13 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-int make_map2(EncodeTiledFn fn, CUtensorMap* map, const float* base, int64_t rows, int64_t row_stride_floats,
-              CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
+int make_map2(EncodeTiledFn fn, CUtensorMap* map, const float* base, int64_t rows, int64_t row_stride_floats) {
     const cuuint64_t dims[2] = {(cuuint64_t)FEAT, (cuuint64_t)rows};
     const cuuint64_t strides[1] = {(cuuint64_t)row_stride_floats * 4};
     const cuuint32_t box[2] = {(cuuint32_t)KBLK, (cuuint32_t)TILE_M};
     const cuuint32_t estr[2] = {1, 1};
     const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     PB_REQUIRE(r == CUDA_SUCCESS, PB_ERR_CUDA, "cuTensorMapEncodeTiled failed: %d", (int)r);
     return PB_OK;
@@ -1239,15 +722,8 @@ int make_map2(EncodeTiledFn fn, CUtensorMap* map, const float* base, int64_t row
 int num_sms() { return pb_num_sms(); }
 
 long long* g_dbg_clk = nullptr;
-int g_update_variant = 2;     // 1 = two x layouts (k_mlp_update_fused), 2 = one x layout + transposing MMA (k_mlp_update_xt)
 
 }  // namespace
-
-extern "C" int pb_mlp_update_set_variant(int32_t variant) {
-    PB_REQUIRE(variant == 1 || variant == 2, PB_ERR_INVALID, "pb_mlp_update_set_variant: 1 or 2");
-    g_update_variant = variant;
-    return PB_OK;
-}
 
 extern "C" int pb_mlp_update_debug_clock(long long* buf) {     // profiling hook: see FusedParams::dbg_clk; nullptr = off
     g_dbg_clk = buf;
@@ -1273,6 +749,8 @@ extern "C" int pb_mlp_update_fused(const float* x, int64_t ldx, int64_t slab_row
                                    int32_t clip_vloss, float vf_clip_coef, float vf_coef, float ent_coef, float* grad_flat,
                                    double* stats8, void* workspace, size_t workspace_bytes, float* dpre_out,
                                    float* dbg_hidden, float* dbg_dpre, float* dbg_dout, void* stream) {
+    PB_REQUIRE(!dpre_out, PB_ERR_UNSUPPORTED,
+               "pb_mlp_update_fused: dpre_out must be NULL (dW_enc is always formed inside the kernel; dPre is not written out)");
     PB_REQUIRE(x && w_enc && b_enc && w_heads && b_heads && actions && old_logprobs && advantages && grad_flat && stats8 &&
                    workspace && (returns || old_values),
                PB_ERR_INVALID, "pb_mlp_update_fused: null pointer");
@@ -1293,9 +771,8 @@ extern "C" int pb_mlp_update_fused(const float* x, int64_t ldx, int64_t slab_row
     const int64_t n_tiles = tiles_per_slab * n_slabs;
     const int64_t map_rows = (int64_t)(n_slabs - 1) * slab_stride_rows + slab_rows;
     PB_REQUIRE(n_tiles <= 0x7FFFFFFF && map_rows <= 0x7FFFFFFF, PB_ERR_UNSUPPORTED, "pb_mlp_update_fused: too many rows");
-    alignas(64) CUtensorMap map_x, map_x32, map_w;
+    alignas(64) CUtensorMap map_x, map_w;
     int rc = make_map2((EncodeTiledFn)fn, &map_x, x, map_rows, ldx);
-    if (rc == PB_OK) rc = make_map2((EncodeTiledFn)fn, &map_x32, x, map_rows, ldx, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
     if (rc == PB_OK) rc = make_map2((EncodeTiledFn)fn, &map_w, w_enc, HID, FEAT);
     if (rc != PB_OK) return rc;
     cudaStream_t s = (cudaStream_t)stream;
@@ -1309,37 +786,19 @@ extern "C" int pb_mlp_update_fused(const float* x, int64_t ldx, int64_t slab_row
     p.part_dw = (float*)workspace; p.part_tail = (float*)workspace + (size_t)num_sms() * FEAT * HID;
     p.dbg_clk = g_dbg_clk;
     p.w_heads = w_heads; p.b_enc = b_enc; p.b_heads = b_heads;
-    p.stats = stats8; p.dpre_out = dpre_out; p.dbg_hidden = dbg_hidden; p.dbg_dpre = dbg_dpre; p.dbg_dout = dbg_dout;
+    p.stats = stats8; p.dbg_hidden = dbg_hidden; p.dbg_dpre = dbg_dpre; p.dbg_dout = dbg_dout;
     PB_CUDA(cudaMemsetAsync(stats8, 0, 8 * sizeof(double), s));
-    if (dpre_out || g_update_variant != 2) {      // variant 1 takes the small operands from the constant bank
-        PB_CUDA(cudaMemcpyToSymbolAsync(c_wh, w_heads, sizeof(float) * NO * HID, 0, cudaMemcpyDeviceToDevice, s));
-        PB_CUDA(cudaMemcpyToSymbolAsync(c_benc, b_enc, sizeof(float) * HID, 0, cudaMemcpyDeviceToDevice, s));
-        PB_CUDA(cudaMemcpyToSymbolAsync(c_bh, b_heads, sizeof(float) * NO, 0, cudaMemcpyDeviceToDevice, s));
-    }
-    // dispatch on the live head rows (n_act + 1: 5 for the 4-action configs, 8 = generic) and on where dW_enc is formed
     static bool attr_set = false;
     if (!attr_set) {
-        PB_CUDA(cudaFuncSetAttribute(k_mlp_update_fused<5, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-        PB_CUDA(cudaFuncSetAttribute(k_mlp_update_fused<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-        PB_CUDA(cudaFuncSetAttribute(k_mlp_update_fused<5, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-        PB_CUDA(cudaFuncSetAttribute(k_mlp_update_fused<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
         PB_CUDA(cudaFuncSetAttribute(k_mlp_update_xt<96, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, X2_TOTAL));
         PB_CUDA(cudaFuncSetAttribute(k_mlp_update_xt<96, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, X2_TOTAL));
         attr_set = true;
     }
-    if (dpre_out) {
-        if (n_act + 1 <= 5) k_mlp_update_fused<5, false><<<grid, THREADS, SMEM_TOTAL, s>>>(map_x, map_x32, map_w, p);
-        else k_mlp_update_fused<8, false><<<grid, THREADS, SMEM_TOTAL, s>>>(map_x, map_x32, map_w, p);
-    } else if (g_update_variant == 2) {
-        // 18 warps = 5 on two of the four schedulers: 16384 registers / (5 x 32) caps the kernel at 96 per thread
-        if (p.dbg_clk) k_mlp_update_xt<96, true><<<grid, X2_THREADS, X2_TOTAL, s>>>(map_x, map_w, p);
-        else k_mlp_update_xt<96, false><<<grid, X2_THREADS, X2_TOTAL, s>>>(map_x, map_w, p);
-    } else {
-        if (n_act + 1 <= 5) k_mlp_update_fused<5, true><<<grid, THREADS, SMEM_TOTAL, s>>>(map_x, map_x32, map_w, p);
-        else k_mlp_update_fused<8, true><<<grid, THREADS, SMEM_TOTAL, s>>>(map_x, map_x32, map_w, p);
-    }
+    // 18 warps = 5 on two of the four schedulers: 16384 registers / (5 x 32) caps the kernel at 96 per thread
+    if (p.dbg_clk) k_mlp_update_xt<96, true><<<grid, X2_THREADS, X2_TOTAL, s>>>(map_x, map_w, p);
+    else k_mlp_update_xt<96, false><<<grid, X2_THREADS, X2_TOTAL, s>>>(map_x, map_w, p);
     PB_LAUNCH_CHECK();
-    k_update_reduce<<<REDUCE_BLOCKS, 256, 0, s>>>(dpre_out ? nullptr : p.part_dw, p.part_tail, grid, grad_flat,
+    k_update_reduce<<<REDUCE_BLOCKS, 256, 0, s>>>(p.part_dw, p.part_tail, grid, grad_flat,
                                                   reinterpret_cast<double*>((char*)workspace + pb_mlp_update_sumsq_offset()));
     PB_LAUNCH_CHECK();
     return PB_OK;

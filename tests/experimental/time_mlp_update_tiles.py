@@ -1,4 +1,4 @@
-"""Per-phase SM-clock stamps of the fused update kernel, variant 2 (pb_mlp_update_debug_clock): where does a tile's time go?
+"""Per-phase SM-clock stamps of the fused update kernel (pb_mlp_update_debug_clock): where does a tile's time go?
 
     python tests/experimental/time_mlp_update_tiles.py
 """
@@ -12,7 +12,6 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 import check_mlp_update_fused as cf      # noqa: E402
 
 lib = cf.lib
-cf._native.check(lib.pb_mlp_update_set_variant(2))
 dev = torch.device('cuda')
 m, n_act = 524288, 4
 torch.manual_seed(0)

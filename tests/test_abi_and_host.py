@@ -52,6 +52,17 @@ def test_calls_fail_loudly_without_a_device():
     assert rc == _native.PB_ERR_CUDA and 'CUDA' in _native.last_error() or 'cuda' in _native.last_error()
 
 
+def test_mlp_update_fused_rejects_dpre_out():
+    """The fused update always forms dW_enc inside the kernel: a non-null dpre_out is refused before anything touches the
+    device, so this holds with or without a GPU."""
+    import ctypes as C
+    p = C.c_void_p(1 << 20)                  # never dereferenced: the argument check comes first
+    rc = _native.lib().pb_mlp_update_fused(p, 128, 128, 128, 1, *[p] * 10, 128, 4, 0.1, 1, 0.1, 0.5, 0.01, p, p, p, 1 << 30,
+                                           p, None, None, None, None)
+    assert rc == _native.PB_ERR_UNSUPPORTED
+    assert 'dpre_out' in _native.last_error()
+
+
 def test_sm100a_only_cubin():
     out = subprocess.check_output(['cuobjdump', '--list-elf', _native.SO_PATH], text=True)
     archs = set(re.findall(r'sm_\d+a?', out))

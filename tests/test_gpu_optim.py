@@ -148,8 +148,7 @@ def test_manual_update_matches_autograd_update():
     assert np.allclose(losses[True], losses[False], rtol=1e-4, atol=1e-6), (losses[True], losses[False])
 
 
-@pytest.mark.parametrize('dw', ['cublas', 'kernel'])
-def test_fused_update_kernel_matches_kernel_chain(dw):
+def test_fused_update_kernel_matches_kernel_chain():
     """train() through pb_mlp_update_fused (ONE tcgen05 kernel per minibatch: csrc/mlp_update.cu) vs the kernel chain it
     replaces (cuBLAS GEMMs + pb_ppo_loss + pb_mlp_tail_backward + split-K dW): same rollout, same minibatches.  Both
     compute the dense products in TF32 (operands truncated by the tensor core), so gradients agree to TF32 noise; the
@@ -165,7 +164,7 @@ def test_fused_update_kernel_matches_kernel_chain(dw):
         vec = pvec.make(ocean.env_creator('breakout'), num_envs=n, backend=pvec.B200)
         torch.manual_seed(0)
         pol = cleanrl.Policy(models.Default(vec.driver_env), fused_sample=True, seed=7).cuda()
-        cfg = make_config(n, h, env='breakout', manual_update=True, fused_update=fused, fused_update_dw=dw)
+        cfg = make_config(n, h, env='breakout', manual_update=True, fused_update=fused)
         cfg.update_epochs = 1
         cfg.minibatch_size = n * h          # ONE minibatch: gflat after train() is its gradient
         data = clean_pufferl.create(cfg, vec, pol)
@@ -199,8 +198,8 @@ def test_fused_update_kernel_matches_kernel_chain(dw):
 
 
 def test_fused_update_kernel_inside_train_graph():
-    """The fused update inside the captured train graph (cudaMemcpyToSymbolAsync nodes + tensor-map kernel parameters)
-    replays to the same parameters as eager execution."""
+    """The fused update inside the captured train graph (tensor-map kernel parameters) replays to the same parameters as
+    eager execution."""
     import pufferlib_b200.vector as pvec
     from pufferlib_b200 import clean_pufferl, models
     from pufferlib_b200.environments import ocean
